@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- FoKL.fit throughput on B200 (BASELINE.json metric: candidate-models/sec; basis-matrix GB/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg4] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg4] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -19,6 +19,9 @@ invocation of the reference (FoKLRoutines.py:1650 / :1681).
     cpu_baseline  the CPU oracle (oracle/fokl_oracle.py, a numpy restatement of the reference) on a bounded sample
 `--impl reference` times that CPU oracle alone (rank 0), same metric / config keys.
 Timing: CUDA events on the launching stream, barrier + synchronize on both sides, max over ranks.
+`--dump-outputs DIR` writes what the last timed resident fit returned (betas, mtx, evs) as DIR/<name>.npy in float64, so
+that two builds can be compared output for output on the same seeded inputs.  Apart from DIR the benchmark writes no
+files: it may run from a read-only tree.
 """
 import argparse
 import json
@@ -55,7 +58,34 @@ def parse():
                     help='--impl reference: total wall-time bound; complete fits are repeated until --steps or this')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-e2e', action='store_true')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write betas / mtx / evs of the last timed fit to DIR/<name>.npy (float64, at most 64 MB)')
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
+    if a.dump_outputs and a.impl != 'b200':
+        ap.error('--dump-outputs writes the device fit: it needs --impl b200')
+    return a
+
+
+DUMP_BYTES = 60 << 20      # array data; keeps the files, headers included, under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> array.  Each is written as out_dir/<name>.npy in float64.  If they would exceed DUMP_BYTES in all,
+    the rows of betas (one per draw) are cut to a sample fixed by seed 0, kept in draw order, so that the files stay
+    comparable between runs."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    over = sum(v.nbytes for v in arrays.values()) - DUMP_BYTES
+    if over > 0:
+        betas = arrays['betas']
+        keep = betas.shape[0] - -(-over // (betas.shape[1] * 8))
+        assert keep > 0, 'the outputs other than betas alone exceed the %d-byte dump budget' % DUMP_BYTES
+        rows = np.sort(np.random.default_rng(0).choice(betas.shape[0], size=keep, replace=False))
+        arrays['betas'] = betas[rows]
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), v)
 
 
 def config_dict(a, n_total, world, extra=None):
@@ -279,6 +309,10 @@ def load_phis(a):
     import warnings
     from FoKL import getKernels
     if bench_data.CONFIGS[a.workload]['kernel'] == 'Cubic Splines':
+        if not os.path.exists(os.path.join(getKernels._KDIR, getKernels.UPSTREAM_SPLINE_FILE)):
+            # the table sp500() would fall back to, built from the current code: no cache file written into the
+            # package, and never one left behind by another build
+            return getKernels._to_phis(getKernels.regenerate_spline_table(500))
         with warnings.catch_warnings():
             warnings.simplefilter('ignore')
             return getKernels.sp500()
@@ -349,11 +383,12 @@ def main():
         return bench_data.make_model(FR, a.workload, draws=a.draws, phis=phis)
 
     ds = eng.upload(x_host, y_host)
+    last_fit = {}
 
     def step_resident():
         np.random.seed(c['seed'])
         model = new_model()
-        model.fit(ds, None)
+        last_fit['betas'], last_fit['mtx'], last_fit['evs'] = model.fit(ds, None)
         return dict(FR.LAST_FIT_INFO)
 
     def step_e2e():
@@ -394,6 +429,8 @@ def main():
     clk = clocks.stop() if rank == 0 else None
     models = sum(i['n_gibbs'] for i in infos)
     value = models / (ms * 1e-3)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, last_fit)
 
     e2e = None
     if not a.no_e2e:

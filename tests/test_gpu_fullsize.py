@@ -144,3 +144,48 @@ def test_cfg3_full_size_properties(phis_bern):
         assert need in sup, (need, sorted(sup))
     assert np.array_equal(evs, evs2)
     FR._engine().release()
+
+
+_DIRECT_FIT = """
+import sys, numpy as np
+sys.path[:0] = [%r, %r]
+import bench_data
+from FoKL import FoKLRoutines as FR, getKernels
+n, draws, out = int(sys.argv[1]), int(sys.argv[2]), sys.argv[3]
+x, y = bench_data.make_rows('cfg4', 0, n, n_total=n)
+phis = getKernels._to_phis(getKernels.regenerate_spline_table(500))
+ds = FR._engine().upload(x, y)
+np.random.seed(bench_data.CONFIGS['cfg4']['seed'])
+betas, mtx, evs = bench_data.make_model(FR, 'cfg4', draws=draws, phis=phis).fit(ds, None)
+np.savez(out, betas=betas, mtx=mtx, evs=evs)
+"""
+
+
+def test_bench_dump_outputs_are_the_last_timed_fit(tmp_path):
+    """bench.py --dump-outputs on a reduced cfg4: the dumped betas / mtx / evs are float64 and equal, bit for bit, to what
+    a direct resident fit of the same seeded data and model returns (in its own process).  --steps 1 and --steps 3 dump
+    the same arrays, and the timed loop really runs that many fits: three times the device launches, the same
+    candidate models per step."""
+    import json
+    import subprocess
+    n, draws = 200000, 200
+    lines, dumps = [], []
+    for steps in (1, 3):
+        d = tmp_path / ('steps%d' % steps)
+        r = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--gpus', '1', '--steps', str(steps),
+                            '--warmup', '1', '--n', str(n), '--draws', str(draws), '--no-cpu-baseline', '--no-e2e',
+                            '--dump-outputs', str(d)], capture_output=True, text=True, timeout=900, cwd=str(tmp_path))
+        assert r.returncode == 0, r.stderr[-3000:]
+        lines.append(json.loads(r.stdout.strip().splitlines()[-1]))
+        dumps.append({k: np.load(str(d / (k + '.npy'))) for k in ('betas', 'mtx', 'evs')})
+    assert lines[1]['gpu_launches'] == 3 * lines[0]['gpu_launches'] > 0
+    assert lines[1]['candidate_models_per_step'] == lines[0]['candidate_models_per_step'] > 0
+    direct = tmp_path / 'direct.npz'
+    r = subprocess.run([sys.executable, '-c', _DIRECT_FIT % (os.path.join(ROOT, 'fokl-gpy_b200'), ROOT), str(n),
+                        str(draws), str(direct)], capture_output=True, text=True, timeout=900, cwd=str(tmp_path))
+    assert r.returncode == 0, r.stderr[-3000:]
+    want = np.load(str(direct))
+    for k in ('betas', 'mtx', 'evs'):
+        for got in dumps:
+            assert got[k].dtype == np.float64 and np.array_equal(got[k], want[k]), k
+    assert want['betas'].shape == (draws, want['mtx'].shape[0] + 1) and want['mtx'].shape[1] == 8

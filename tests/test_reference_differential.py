@@ -2,7 +2,8 @@
 `evaluate_basis`, constructor / `clear` / `save` / `load`, `evaluate` / `coverage3` on a hand-made model with the device
 product replaced by numpy, the error paths) run on the UNMODIFIED reference and on this
 package, outcome by outcome -- returned values bit-identical, same attributes, same exception type, same warning
-texts.  The reference lives only in the build container (/root/reference); elsewhere the test is skipped."""
+texts.  The reference is not part of this repository: the tests run where oracle/ref_harness.py finds its sources
+(FOKL_REFERENCE_SRC names the src/ directory of an unmodified upstream FoKL-GPy checkout) and are skipped elsewhere."""
 import os
 import pickle
 import subprocess
@@ -13,7 +14,10 @@ import pytest
 
 from conftest import ROOT
 
-REF_SRC = '/root/reference/src'
+from ref_harness import REF_SRC
+
+needs_reference = pytest.mark.skipif(not os.path.isdir(REF_SRC),
+                                     reason='needs the upstream FoKL-GPy sources: set FOKL_REFERENCE_SRC')
 CASES = os.path.join(ROOT, 'tests', 'diff', 'host_api_cases.py')
 
 
@@ -52,7 +56,7 @@ DEPARTURES = {
 }
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason='the reference is only present in the build container')
+@needs_reference
 def test_host_api_outcomes_equal_the_reference(tmp_path):
     ref = _run([os.path.join(ROOT, 'oracle', '_stubs'), REF_SRC, os.path.join(ROOT, 'oracle')], str(tmp_path / 'ref.pkl'))
     mine = _run([os.path.join(ROOT, 'fokl-gpy_b200'), os.path.join(ROOT, 'oracle'), os.path.join(ROOT, 'tests')],
@@ -74,7 +78,7 @@ def test_host_api_outcomes_equal_the_reference(tmp_path):
     assert not bad, '\n'.join('%s [%s]\n  reference: %.300r\n  here:      %.300r' % b for b in bad)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason='the reference is only present in the build container')
+@needs_reference
 def test_small_fits_with_unusual_hypers_equal_the_live_reference(tmp_path, monkeypatch):
     """28 small whole fits (Bernoulli and cubic kernels, raw inputs, clean=True) with the hyper-parameters the golden fixtures do not
     reach -- gimmie, aic, tolerance 1 / 5, loose / tight kill thresholds, strong / weak priors, hyper-parameters passed
@@ -122,7 +126,7 @@ def test_small_fits_with_unusual_hypers_equal_the_live_reference(tmp_path, monke
     assert not bad, bad
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason='the reference is only present in the build container')
+@needs_reference
 def test_oracle_equals_the_live_reference_on_the_small_fits(tmp_path, phis_cubic, phis_bern):
     """The checker itself: oracle/fokl_oracle.py `fit` on the reference's own cleaned train set and resolved
     hyper-parameters, for the same configurations -- term matrix, numpy RNG end state and returned draws identical,
@@ -167,7 +171,7 @@ def test_oracle_equals_the_live_reference_on_the_small_fits(tmp_path, phis_cubic
     assert checked >= 26
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason='the reference is only present in the build container')
+@needs_reference
 def test_update_flows_equal_the_live_reference(tmp_path, monkeypatch):
     """Five update flows (`update = True`; `clean` with a fixed minmax, `fit()`, next batch, `fit()` -- the way
     examples/sigmoid/updateSig.py drives it) with both kernels, aic, gimmie, tolerance 1 / 2, on the live reference and
