@@ -684,8 +684,10 @@ __global__ void __launch_bounds__(32 * kStatsRows) cand_stats_kernel(const Stats
     __syncthreads();
     s0 = 0.0; s1 = 0.0;
     for (int r = 0; r < kStatsRows; ++r) { s0 += red[0][r][tx]; s1 += red[1][r][tx]; }
+    // a window that starts at or after row D (D <= 3 with the windows of FR:1656-1658) is empty: its mean and standard
+    // deviation are NaN, as numpy's of an empty slice
     const double n0 = (double)(P.D - P.from0), n1 = (double)(P.D - P.from1);
-    const double m0 = s0 / n0, m1 = s1 / n1;
+    const double m0 = n0 > 0.0 ? s0 / n0 : nan(""), m1 = n1 > 0.0 ? s1 / n1 : nan("");
     double q = 0.0;
     if (on)
         for (int k = P.from1 + ty; k < P.D; k += kStatsRows) {
@@ -700,7 +702,7 @@ __global__ void __launch_bounds__(32 * kStatsRows) cand_stats_kernel(const Stats
         for (int r = 0; r < kStatsRows; ++r) q += red[0][r][tx];
         double *S = P.stats + 3 * m.vec_off;
         S[i] = m1;
-        S[p + i] = sqrt(q / n1);
+        S[p + i] = n1 > 0.0 ? sqrt(q / n1) : nan("");
         S[2 * p + i] = m0;
     }
 }
@@ -1102,8 +1104,9 @@ extern "C" int fokl_candidates_eval(fokl_ctx *ctx, const double *G, int64_t ldg,
     const bool philox = rng_mode == FOKL_RNG_PHILOX;
     double *d_gam = nullptr, *d_var = nullptr, *d_betas = nullptr, *d_sigs = nullptr, *d_taus = nullptr;
     if (n_chain > 0) {
-        if (hyp->stat_from0 < 0 || hyp->stat_from0 >= D || hyp->stat_from1 < 0 || hyp->stat_from1 >= D)
-            FOKL_FAIL(ctx, FOKL_EINVAL, "candidates_eval: statistic windows outside the chain");
+        // a window may start at or after row D (an empty window: NaN statistics), never before row 0
+        if (hyp->stat_from0 < 0 || hyp->stat_from1 < 0)
+            FOKL_FAIL(ctx, FOKL_EINVAL, "candidates_eval: negative statistic window start");
         size_t c_bytes = 256 + ((size_t)D * gam + (philox ? (size_t)D * (gam + 2 * (size_t)n_chain) : 0)) * sizeof(double);
         char *ccur = (char *)fokl_scratch(ctx, fokl_ctx::B_CAND_C, c_bytes);
         if (!ccur) return FOKL_ENOMEM;

@@ -162,7 +162,7 @@ typedef struct fokl_hypers {
  * Outputs (dev; any of betahat/lamb/Q/betas/sigs/taus/stats may be NULL):
  *   ev[c]        BIC (FR:1554), without the aic adjustment (FR:1654, host side)
  *   stats        per candidate 3 x p_c: row 0 mean over rows [stat_from1, D), row 1 std (ddof 0) over the
- *                same rows, row 2 mean over rows [stat_from0, D)
+ *                same rows, row 2 mean over rows [stat_from0, D); NaN over an empty window (start >= D, D <= 3)
  *   info[c]      bit 0: bstar < 0 seen (FR:1538); bits 8..: Jacobi sweeps used                      */
 int fokl_candidates_eval(fokl_ctx *ctx, const double *G, int64_t ldg, const double *Xty,
                          const int32_t *col_sets, const int32_t *set_offsets, int n_cand,
