@@ -68,6 +68,7 @@ PROTOTYPES = {
     'fokl_fill_ones': (_i32, [_vp, _vp, _i64]),
     'fokl_gram_update': (_i32, [_vp, _vp, _i64, _i64, _i32, _i32, _vp, _vp]),
     'fokl_gram_update_ex': (_i32, [_vp, _vp, _i64, _i64, _i32, _i32, _i32, _i32, _vp, _vp]),
+    'fokl_gram_last_config': (_i32, [_vp, _vp]),
     'fokl_y_moments': (_i32, [_vp, _vp, _i64, _vp]),
     'fokl_gram_scatter': (_i32, [_vp, _vp, _i32, _i32, _vp, _i64, _vp]),
     'fokl_gram_compact': (_i32, [_vp, _vp, _i64, _vp, _vp, _i32, _vp, _i64, _vp]),

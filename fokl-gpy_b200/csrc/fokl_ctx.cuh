@@ -18,6 +18,8 @@ struct fokl_ctx {
     bool own_stream = false;
     std::string err;
     int64_t launches = 0;
+    // what the last fokl_gram_update(_ex) launched (fokl_gram_last_config); gram_cfg[0] < 0: none yet
+    int64_t gram_cfg[9] = {-1, 0, 0, 0, 0, 0, 0, 0, 0};
     int num_sms = 148;
     int sm_budget = 0;        // > 0: SMs a batch of candidate models may plan for (fokl_ctx_set_sm_budget)
     size_t smem_optin = 0;

@@ -784,6 +784,15 @@ bool encode_gram_map(CUtensorMap *map, const double *base, int64_t ld, int64_t n
 
 }  // namespace
 
+extern "C" int fokl_gram_last_config(fokl_ctx *ctx, int64_t out[9])
+{
+    FOKL_CHECK_CTX(ctx);
+    if (!out) FOKL_FAIL(ctx, FOKL_EINVAL, "gram_last_config: bad argument");
+    if (ctx->gram_cfg[0] < 0) FOKL_FAIL(ctx, FOKL_ESTATE, "gram_last_config: no Gram update on this context yet");
+    memcpy(out, ctx->gram_cfg, sizeof ctx->gram_cfg);
+    return FOKL_OK;
+}
+
 extern "C" int fokl_gram_update(fokl_ctx *ctx, const double *X, int64_t ld, int64_t n, int p_old, int c,
                                 const double *y, double *block)
 {
@@ -953,6 +962,9 @@ extern "C" int fokl_gram_update_ex(fokl_ctx *ctx, const double *X, int64_t ld, i
     P.part = reinterpret_cast<double *>(buf + part_off);
     P.n_tiles = n_tiles;
     P.tile_blocks = kTileBlocks;
+    const int64_t cfg[9] = {use_tma ? 2 : (use_mb ? 1 : 0), warps, kb, stages, n_tiles, nsplit, rows_per_split,
+                            plan.max_slots, cap};
+    memcpy(ctx->gram_cfg, cfg, sizeof cfg);
     const size_t smem = use_tma ? smem_need_tma(plan.max_slots, kb, stages) : smem_need(plan.max_slots, kb, stages);
     if (use_tma) {
         GramTmaMaps maps;

@@ -114,6 +114,11 @@ int fokl_gram_update(fokl_ctx *ctx, const double *X, int64_t ld, int64_t n, int 
 #define FOKL_GRAM_CROSS_ONLY 1
 int fokl_gram_update_ex(fokl_ctx *ctx, const double *X, int64_t ld, int64_t n, int p_old, int c, int new_col0,
                         int flags, const double *y, double *block);
+/* what the last fokl_gram_update(_ex) on this context launched (host record, for tests and tuning):
+ * out (host, 9 values) = { pipeline (0 = cp.async ring, 1 = bulk-copy / mbarrier ring, 2 = tensor-map ring),
+ * consumer warps, rows per slab (kb), ring stages, tiles, row splits, rows per split, staged-column slots per tile,
+ * slot cap }.  FOKL_ESTATE if the context has not launched one yet. */
+int fokl_gram_last_config(fokl_ctx *ctx, int64_t out[9]);
 
 /* moments of y: out (dev, 3 doubles) = { n, sum y, sum y^2 } (dtd, FR:1374). */
 int fokl_y_moments(fokl_ctx *ctx, const double *y, int64_t n, double *out);

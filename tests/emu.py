@@ -55,7 +55,7 @@ def lib():
     L.emu_philox_normals.restype = None
     L.emu_philox_gammas.argtypes = [_u64, _u64, _i32, _f64, _vp]
     L.emu_philox_gammas.restype = None
-    L.emu_gram_plan.argtypes = [_vp, _i64, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp]
+    L.emu_gram_plan.argtypes = [_vp, _i64] + [_i32] * 11 + [_vp, _vp, _vp]
     L.emu_gram_plan.restype = _i32
     L.emu_update_chain.argtypes = [_vp] * 13 + [_u64, _u64] + [_vp] * 5
     L.emu_update_chain.restype = _i32
@@ -169,20 +169,32 @@ def kill_loop(G, Xty, idx, cand_pos, bv0, bv1, hyp, threshav=0.05, threshstda=0.
                 calls=out_i[3 + vm:3 + vm + k].copy(), ev=out_ev[:k].copy())
 
 
-def gram_plan(A, p_old, c, cap=352, warps=16, kchunks=1, mode=1):
-    """Walk the K2 work plan on the host (slabs of kchunks 16-row chunks): returns (block (p + 1) x c with NaN where
-    nothing was written, cover counts, stats dict)."""
-    A = np.ascontiguousarray(A, dtype=np.float64)
-    n, p1 = A.shape
-    assert p1 == p_old + c + 1
+_GRAM_STATS = ('n_tiles', 'max_slots', 'blocks', 'max_positions_per_tile', 'max_ksplit', 'sp_spread', 'flex_late', 'pad',
+               'loose', 'flex0', 'flex1', 'flex2', 'min_ksplit', 'box8', 'box32', 'box128', 'max_runs')
+
+
+def gram_plan(A, p_old, c, cap=352, warps=16, kchunks=1, mode=1, gap=0, cross_only=False, allow_loose=True, pad_mode=-1,
+              force_r=0):
+    """Walk the K2 work plan on the host (slabs of kchunks 16-row chunks): returns (rc, block (p + 1) x c with NaN where
+    nothing was written, cover counts, stats dict).  A: [n][p_old + gap + c + 1] in the physical column order of
+    fokl_gram_update_ex (old | gap | new | y), or None for the plan checks and statistics alone.  stats: tiles, slots
+    and blocks, the k-split range, the pad layout chosen, loose items, busy warps in each consumer form (flex0/1/2),
+    tensor-map boxes of each kind and the longest run table of the bulk-copy kernel."""
+    p1 = p_old + c + 1
+    if A is None:
+        n, ptr = 0, None
+    else:
+        A = np.ascontiguousarray(A, dtype=np.float64)
+        n = A.shape[0]
+        assert A.shape[1] == p1 + gap
+        ptr = A.ctypes.data
     out = np.full((p1, c), np.nan)
     cover = np.zeros((p1, c), dtype=np.int32)
-    stats = np.zeros(7, dtype=np.int32)
-    rc = lib().emu_gram_plan(A.ctypes.data, n, p_old, c, cap, warps, kchunks, mode, out.ctypes.data, cover.ctypes.data,
+    stats = np.zeros(len(_GRAM_STATS), dtype=np.int32)
+    rc = lib().emu_gram_plan(ptr, n, p_old, c, cap, warps, kchunks, mode, gap, int(bool(cross_only)),
+                             int(bool(allow_loose)), pad_mode, force_r, out.ctypes.data, cover.ctypes.data,
                              stats.ctypes.data)
-    return rc, out, cover, dict(n_tiles=int(stats[0]), max_slots=int(stats[1]), blocks=int(stats[2]),
-                                max_positions_per_tile=int(stats[3]), max_ksplit=int(stats[4]), sp_spread=int(stats[5]),
-                                flex_late=int(stats[6]))
+    return rc, out, cover, {k: int(v) for k, v in zip(_GRAM_STATS, stats)}
 
 
 def update_chain(mode, po, pn, draws, astar, atau_star, b, btau, sigsqd0, yty, squerr, n, arrays, variates=None, seed=0,

@@ -237,29 +237,51 @@ int emu_update_chain(const int32_t *mdl, const double *par, const double *lam_o,
 
 }  // extern "C"
 
-// ---- K2 work plan (csrc/gram_plan.h): host walk of tiles / blocks / fragments exactly as gram_kernel +
-// gram_reduce_kernel use them.  A is [n][p + 1] row-major with y as the last column; out is (p + 1) x c and must be
-// pre-filled by the caller; cover (same shape, int) counts how many times each entry was written.
+// ---- K2 work plan (csrc/gram_plan.h): host walk of tiles / blocks / fragments exactly as the Gram kernels +
+// gram_reduce_kernel use them.  A is [n][p + gap + 1] row-major in the PHYSICAL column order of fokl_gram_update_ex
+// (old columns, `gap` unused columns, new columns, y last) and may be null (plan checks and statistics only); out is
+// (p + 1) x c in the logical order old | new | y and must be pre-filled by the caller; cover (same shape, int) counts
+// how many times each entry was written.  pad_mode -1 / allow_loose 1 / force_r 0 are the defaults of gram_make_plan
+// and gram_plan_place.
 #include "../../fokl-gpy_b200/csrc/gram_plan.h"
-extern "C" int emu_gram_plan(const double *A, int64_t n, int p_old, int c, int max_slots_cap, int warps, int kchunks, int mode, double *out,
-                             int32_t *cover, int32_t *stats /* n_tiles, max_slots, total_blocks, max_positions_per_tile, max_ksplit, sp_spread, flex_late */)
+extern "C" int emu_gram_plan(const double *A, int64_t n, int p_old, int c, int max_slots_cap, int warps, int kchunks, int mode,
+                             int gap, int cross_only, int allow_loose, int pad_mode, int force_r, double *out, int32_t *cover,
+                             int32_t *stats /* see kGramStats below */)
 {
+    // stats: 0 n_tiles, 1 max_slots, 2 total_blocks, 3 max_positions_per_tile, 4 max_ksplit, 5 sp_spread, 6 flex_late,
+    // 7 pad layout, 8 loose items, 9-11 warps in FLEX form 0 / 1 / 2, 12 min_ksplit, 13-15 boxes of 8 / 32 / 128 columns,
+    // 16 largest run count of the bulk-copy kernel's run table in one tile
     const int p = p_old + c;
-    GramPlan pl = gram_make_plan(p_old, c, max_slots_cap, warps);
-    gram_plan_place(pl, warps, kchunks, mode);
+    const int W = p + gap + 1;                       // columns of A
+    auto logical = [&](int src) { return src < 0 ? -1 : (src >= p_old + gap ? src - gap : src); };
+    GramPlan pl = gram_make_plan(p_old, c, max_slots_cap, warps, gap, cross_only != 0, pad_mode, allow_loose != 0);
+    int pad_used = pad_mode;
+    if (pad_used < 0) {
+        // the layout the default chose: rebuild both and compare
+        pad_used = 0;
+        if (((c + 7) / 8) % 2 == 1) {
+            GramPlan b = gram_make_plan(p_old, c, max_slots_cap, warps, gap, cross_only != 0, 1, allow_loose != 0);
+            if (b.slot_src == pl.slot_src && b.blocks.size() == pl.blocks.size()) pad_used = 1;
+        }
+    }
+    gram_plan_place(pl, warps, kchunks, mode, force_r);
     const int kTileBlocks = gram_tile_blocks(warps);
+    for (int k = 0; k < 17; ++k) stats[k] = 0;
     stats[0] = (int32_t)pl.tiles.size();
     stats[1] = pl.max_slots;
-    stats[2] = 0;
-    stats[3] = 0;
-    stats[4] = 0;
-    stats[5] = 0;       // largest spread of items over the sub-partitions that still have room
-    stats[6] = 0;       // loose / masked items placed behind a warp's first position although every busy warp could take one
+    stats[7] = pad_used;
+    stats[12] = 1 << 30;
     for (const GramTileMeta &tm : pl.tiles) {
         if (tm.n_blk > stats[3]) stats[3] = tm.n_blk;
         if (tm.ksplit > stats[4]) stats[4] = tm.ksplit;
+        if (tm.ksplit < stats[12]) stats[12] = tm.ksplit;
         if (tm.n_blk > kTileBlocks || tm.n_slots > max_slots_cap || (tm.n_slots % 8) != 0) return -1;
         if (tm.ksplit < 1 || tm.ksplit > kchunks || (kchunks % tm.ksplit) != 0) return -5;
+        for (int s = 0; s < tm.n_slots; ++s) {
+            const int src = pl.slot_src[tm.slot_off + s];
+            if (src < -1 || src >= W || (src >= p_old && src < p_old + gap)) return -10;     // never a gap column
+            if (logical(src) != pl.slot_arow[tm.slot_off + s]) return -10;
+        }
         // positions of a warp are filled from its first one (the kernel stops at the first hole)
         for (int w = 0; w < warps; ++w) {
             bool hole = false;
@@ -272,19 +294,25 @@ extern "C" int emu_gram_plan(const double *A, int64_t n, int p_old, int c, int m
             }
             if (owned > gram_warp_cap(warps, w)) return -8;
         }
-        // placement statistics: items per SM sub-partition (warp & 3), loose / masked items outside a warp's first position
+        // placement statistics: items per SM sub-partition (warp & 3), loose / masked items outside a warp's first
+        // position, the consumer form of every busy warp (gram_kernel_mb / gram_kernel_tma: FLEX)
         {
             int sl[4] = {0, 0, 0, 0}, busy = 0, flex_total = 0, flex_late = 0;
             for (int w = 0; w < warps; ++w) {
-                int owned = 0;
-                for (int q = w, b = 0; q < tm.n_blk; q += warps, ++b) {
+                int owned = 0, flex = 0;
+                for (int q = w, b = 0; q < tm.n_blk && b < kGramBlocksPerWarp; q += warps, ++b) {
                     const GramBlockMeta &bm = pl.blocks[tm.blk_off + q];
                     if (bm.mask == 0) break;
                     ++owned;
-                    if (bm.loose || bm.mask != 15) { ++flex_total; flex_late += b > 0; }
+                    if (bm.loose || bm.mask != 15) {
+                        ++flex_total;
+                        flex_late += b > 0;
+                        flex = b == 0 ? (flex > 1 ? flex : 1) : 2;
+                    }
                 }
                 sl[w & 3] += owned;
                 busy += owned > 0;
+                if (owned > 0) ++stats[9 + flex];
             }
             int mx = 0, mn = 1 << 30;
             for (int q = 0; q < 4; ++q) {
@@ -296,11 +324,43 @@ extern "C" int emu_gram_plan(const double *A, int64_t n, int p_old, int c, int m
             if (mn != (1 << 30) && mx - mn > stats[5]) stats[5] = mx - mn;
             if (flex_total <= busy) stats[6] += flex_late;
         }
-        // gram_kernel: every item accumulates its own chunks; gram_reduce_kernel: the head walks the chain
+        // the bulk-copy kernel's run table (gram_kernel_mb): same walk
+        {
+            int n_runs = 0, prev = -2;
+            for (int sl = 0; sl < tm.n_slots; ++sl) {
+                const int src = pl.slot_src[tm.slot_off + sl];
+                if (src < 0) { prev = -2; continue; }
+                if (!(src == prev + 1 && src != p + gap && n_runs > 0)) ++n_runs;
+                prev = src;
+            }
+            if (n_runs > stats[16]) stats[16] = n_runs;
+        }
+        // TMA boxes: inside the tile, every non-padding slot fetched exactly once from its own column of [y | X]
+        {
+            auto xcol = [&](int src) { return src == p + gap ? 0 : src + 1; };
+            std::vector<int> got(tm.n_slots, 0);
+            for (int b = 0; b < tm.n_box; ++b) {
+                const GramBoxMeta &bx = pl.boxes[tm.box_off + b];
+                if (bx.kind < 0 || bx.kind >= kGramBoxKinds || bx.ncols != kGramBoxCols[bx.kind]) return -11;
+                if (bx.slot0 < 0 || bx.slot0 % 8 != 0 || bx.slot0 + bx.ncols > tm.n_slots) return -11;
+                ++stats[13 + bx.kind];
+                for (int i = 0; i < bx.ncols; ++i) {
+                    const int src = pl.slot_src[tm.slot_off + bx.slot0 + i];
+                    if (src < 0) continue;
+                    if (xcol(src) != bx.xcol0 + i) return -12;
+                    ++got[bx.slot0 + i];
+                }
+            }
+            for (int s = 0; s < tm.n_slots; ++s)
+                if (got[s] != (pl.slot_src[tm.slot_off + s] >= 0 ? 1 : 0)) return -13;
+        }
+        // the kernels: every item accumulates its own chunks; gram_reduce_kernel: the head walks the chain
         std::vector<double> part((size_t)tm.n_blk * 256, 0.0);
         for (int q = 0; q < tm.n_blk; ++q) {
             const GramBlockMeta bm = pl.blocks[tm.blk_off + q];
             if (bm.mask == 0) continue;
+            if (bm.loose) ++stats[8];
+            if (bm.loose && !allow_loose) return -9;
             for (int f = 0; f < 4; ++f)
                 if (bm.la[f] + 8 > tm.n_slots || bm.lb[f] + 8 > tm.n_slots) return -2;
             if (!bm.loose)
@@ -309,6 +369,7 @@ extern "C" int emu_gram_plan(const double *A, int64_t n, int p_old, int c, int m
             if (bm.mask > 15 || bm.phase >= tm.ksplit) return -4;
             if (bm.next >= tm.n_blk || (bm.next >= 0 && pl.blocks[tm.blk_off + bm.next].phase != bm.phase + 1)) return -7;
             if ((bm.next < 0) != (bm.phase == tm.ksplit - 1)) return -7;
+            if (!A) continue;
             for (int f = 0; f < 4; ++f)
                 for (int idx = 0; idx < 64; ++idx) {
                     if (!(bm.mask >> f & 1)) continue;
@@ -317,7 +378,7 @@ extern "C" int emu_gram_plan(const double *A, int64_t n, int p_old, int c, int m
                     if (ca < 0 || cb < 0) continue;
                     double s = 0.0;
                     for (int64_t i = 0; i < n; ++i)
-                        if ((int)((i / 16) % tm.ksplit) == bm.phase) s += A[i * (p + 1) + ca] * A[i * (p + 1) + cb];
+                        if ((int)((i / 16) % tm.ksplit) == bm.phase) s += A[i * W + ca] * A[i * W + cb];
                     part[(size_t)q * 256 + f * 64 + idx] = s;
                 }
         }
@@ -332,7 +393,7 @@ extern "C" int emu_gram_plan(const double *A, int64_t n, int p_old, int c, int m
                     const int sb = tm.slot_off + bm.lb[f] + (idx & 7);
                     const int arow = pl.slot_arow[sa], bcol = pl.slot_bcol[sb];
                     if (arow < 0 || bcol < 0) continue;
-                    const int ca = pl.slot_src[sa], cb = pl.slot_src[sb];
+                    const int ca = logical(pl.slot_src[sa]), cb = logical(pl.slot_src[sb]);
                     if (ca != arow || cb != p_old + bcol || cb >= p) return -3;
                     double s = 0.0;
                     int links = 0;

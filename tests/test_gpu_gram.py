@@ -1,69 +1,9 @@
-"""K2 (fokl_gram_update + scatter/compact) against numpy: rtol 1e-12 (summation order differs from OpenBLAS)."""
+"""K2 inside the engine: G / Xty after appends, compactions and the build-ahead layout against numpy (rtol 1e-12).
+The kernels themselves are compared with exact and long-double references in tests/test_gpu_gram_ref.py."""
 import numpy as np
 import pytest
 
 pytestmark = pytest.mark.gpu
-
-
-def gram_block(engine, Xh, yh, p_old, c, joint=False):
-    """joint: y stored in the row in front of X (the engine's [y | X] buffer -> tensor-map TMA kernel); otherwise y is
-    a separate buffer (mbarrier / cp.async kernels)."""
-    import torch
-    n, p = Xh.shape
-    ld = ((n + 15) // 16) * 16
-    full = torch.zeros((p + 1, ld), dtype=torch.float64, device=engine.device)
-    X = full[1:]
-    X[:, :n] = torch.from_numpy(np.ascontiguousarray(Xh.T)).to(engine.device)
-    if joint:
-        y = full[0]
-        # rows n .. ld of the buffer are never read as data: poison them
-        full[:, n:] = float('nan')
-    else:
-        y = torch.zeros(ld, dtype=torch.float64, device=engine.device)
-    y[:n] = torch.from_numpy(yh).to(engine.device)
-    block = torch.full(((p_old + c + 1) * c,), np.nan, dtype=torch.float64, device=engine.device)
-    engine._ck(engine.lib.fokl_gram_update(engine.ctx, X.data_ptr(), ld, n, p_old, c, y.data_ptr(), block.data_ptr()))
-    engine.synchronize()
-    return block.cpu().numpy().reshape(p_old + c + 1, c)
-
-
-@pytest.mark.parametrize('joint', [False, True])
-@pytest.mark.parametrize('n,p_old,c', [(1, 1, 1), (10, 1, 2), (33, 3, 5), (1000, 9, 8), (4097, 63, 1), (4097, 64, 64),
-                                        (2500, 65, 67), (100000, 130, 40), (300001, 20, 168)])
-def test_gram_block_matches_numpy(engine, n, p_old, c, joint, monkeypatch):
-    if joint:       # every shape through the tensor-map kernel (the library would pick it for wide tiles only)
-        monkeypatch.setenv('FOKL_GRAM_KERNEL', 'tma')
-    rng = np.random.default_rng(n + p_old)
-    Xh = rng.standard_normal((n, p_old + c))
-    Xh[:, 0] = 1.0
-    yh = rng.standard_normal(n)
-    got = gram_block(engine, Xh, yh, p_old, c, joint)
-    A = np.hstack([Xh, yh[:, None]])
-    ref = A.T @ Xh[:, p_old:]
-    scale = np.sqrt(np.outer(np.sum(A * A, axis=0), np.sum(Xh[:, p_old:] ** 2, axis=0)))
-    ok = np.abs(got - ref) <= 1e-12 * scale + 1e-300
-    # entries strictly below the diagonal of the symmetric X_new' X_new part are optional: the kernel skips 8 x 8
-    # fragments that lie entirely there (they read back as 0) and fokl_gram_scatter mirrors the upper triangle
-    a, j = np.meshgrid(np.arange(p_old + c + 1) - p_old, np.arange(c), indexing='ij')
-    below = (a > j) & (a < c)
-    assert np.all(ok | (below & (got == 0.0)))
-    assert np.all(ok[~below])
-    # deterministic: a second run gives identical bits
-    again = gram_block(engine, Xh, yh, p_old, c, joint)
-    assert np.array_equal(got, again)
-    # scattered into the master Gram the block is exactly symmetric and complete
-    import torch
-    P = p_old + c
-    G = torch.zeros((P, P), dtype=torch.float64, device=engine.device)
-    Xty = torch.zeros(P, dtype=torch.float64, device=engine.device)
-    blk = torch.from_numpy(got.reshape(-1)).to(engine.device)
-    engine._ck(engine.lib.fokl_gram_scatter(engine.ctx, blk.data_ptr(), p_old, c, G.data_ptr(), P, Xty.data_ptr()))
-    Gh = G.cpu().numpy()
-    full = Xh.T @ Xh
-    assert np.array_equal(Gh[:, p_old:], Gh[p_old:, :].T)
-    sc = np.sqrt(np.outer(np.diag(full), np.diag(full)))
-    assert np.all(np.abs(Gh[:, p_old:] - full[:, p_old:]) <= 1e-12 * sc[:, p_old:])
-    assert np.allclose(Xty.cpu().numpy()[p_old:], Xh[:, p_old:].T @ yh, rtol=1e-10, atol=1e-9)
 
 
 def test_engine_gram_state_append_and_compact(engine, phis_cubic):
@@ -97,50 +37,6 @@ def test_engine_gram_state_append_and_compact(engine, phis_cubic):
     assert np.array_equal(engine.Xty[:5].cpu().numpy(), Xty[keep])
     Xd = engine.X[:5, :n].t().cpu().numpy()
     assert np.array_equal(Xd, Xh[:, keep])
-
-
-@pytest.mark.parametrize('joint', [False, True])
-@pytest.mark.parametrize('n,p_old,c,gap', [(10, 1, 2, 3), (2500, 65, 67, 9), (100000, 30, 40, 168), (300001, 20, 168, 56)])
-def test_gram_block_with_gap_and_cross_only(engine, n, p_old, c, gap, joint, monkeypatch):
-    """fokl_gram_update_ex: the new block stored `gap` columns above the old ones (built ahead of time, above columns
-    the previous substage may still delete -- here poisoned with NaN) gives the SAME BITS as the contiguous layout;
-    FOKL_GRAM_CROSS_ONLY leaves the new x new rows zero and reproduces the (old | y) x new rows bit for bit."""
-    import torch
-    from FoKL import _lib
-    if joint:
-        monkeypatch.setenv('FOKL_GRAM_KERNEL', 'tma')
-    rng = np.random.default_rng(n + p_old + gap)
-    Xh = rng.standard_normal((n, p_old + c))
-    Xh[:, 0] = 1.0
-    yh = rng.standard_normal(n)
-    ref = gram_block(engine, Xh, yh, p_old, c, joint)
-    ld = ((n + 15) // 16) * 16
-    full = torch.full((p_old + gap + c + 1, ld), float('nan'), dtype=torch.float64, device=engine.device)
-    full[:, :n] = 0.0
-    X = full[1:]
-    X[:p_old, :n] = torch.from_numpy(np.ascontiguousarray(Xh[:, :p_old].T)).to(engine.device)
-    X[p_old:p_old + gap, :n] = float('nan')                      # dead columns: never read as data
-    X[p_old + gap:, :n] = torch.from_numpy(np.ascontiguousarray(Xh[:, p_old:].T)).to(engine.device)
-    if joint:
-        y = full[0]
-    else:
-        y = torch.zeros(ld, dtype=torch.float64, device=engine.device)
-    y[:n] = torch.from_numpy(yh).to(engine.device)
-    for flags in (0, _lib.GRAM_CROSS_ONLY):
-        block = torch.full(((p_old + c + 1) * c,), np.nan, dtype=torch.float64, device=engine.device)
-        engine._ck(engine.lib.fokl_gram_update_ex(engine.ctx, X.data_ptr(), ld, n, p_old, c, p_old + gap, flags,
-                                                  y.data_ptr(), block.data_ptr()))
-        engine.synchronize()
-        got = block.cpu().numpy().reshape(p_old + c + 1, c)
-        if flags == 0:
-            assert np.array_equal(got, ref)
-        else:
-            # another plan (fewer blocks per tile, another k-split): same values to rounding, not the same bits
-            A = np.hstack([Xh[:, :p_old], yh[:, None]])
-            scale = np.sqrt(np.outer(np.sum(A * A, axis=0), np.sum(Xh[:, p_old:] ** 2, axis=0)))
-            rows = list(range(p_old)) + [p_old + c]
-            assert np.all(np.abs(got[rows] - ref[rows]) <= 1e-12 * scale)
-            assert np.all(got[p_old:p_old + c] == 0.0)
 
 
 def test_engine_build_ahead_layout(engine, phis_cubic):

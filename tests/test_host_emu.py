@@ -267,6 +267,86 @@ def test_gram_k_split_fills_the_cta():
     assert rc == 0 and st['max_ksplit'] == 1
 
 
+GRAM_SHAPES = [(0, 1), (1, 1), (1, 7), (1, 8), (1, 9), (7, 16), (8, 17), (9, 24), (16, 33), (50, 8), (14, 56), (1, 146),
+               (28, 168), (58, 168), (130, 40), (20, 300), (400, 17)]
+# plan forms the kernels run: (consumer warps, kchunks, placement mode, loose items, forced pad layout, forced k-split)
+GRAM_FORMS = {
+    'mb15-place2': (15, 16, 2, True, -1, 0),
+    'tma12-place2': (12, 16, 2, True, -1, 0),
+    'cpasync16': (16, 1, 2, False, -1, 0),
+    'place0-pad0-ks2': (15, 4, 0, True, 0, 2),
+    'place1-pad1-ks16': (15, 16, 1, True, 1, 16),
+}
+
+
+@pytest.mark.parametrize('form', list(GRAM_FORMS))
+@pytest.mark.parametrize('p_old,c', GRAM_SHAPES)
+def test_gram_plan_forms_cover_the_block_exactly_once(p_old, c, form):
+    """Every plan form of K2 -- the cp.async plan (no loose items), both pad layouts, forced k-splits, placements 0 / 1 /
+    2, 12 and 15 warps -- contiguous, with the new block `gap` columns above the old ones (physical slot_src: the same
+    logical block, the same bits) and cross-only (the new x new rows are not produced).  Inside emu_gram_plan: every
+    tensor-map box lies inside its tile and fetches each non-padding slot exactly once from its own column of [y | X];
+    the bulk-copy kernel's run table (max_slots * 8 bytes = max_slots / 2 runs) is never overrun."""
+    warps, kchunks, mode, loose, pad, force_r = GRAM_FORMS[form]
+    cap = 352
+    rng = np.random.default_rng(p_old * 1000 + c)
+    n = 16 * 2 * kchunks + 5
+    p = p_old + c
+    A = rng.standard_normal((n, p + 1))
+    ref = A.T @ A[:, p_old:p]
+    a, j = np.meshgrid(np.arange(p + 1) - p_old, np.arange(c), indexing='ij')
+    new = (a >= 0) & (a < c)
+    needed = ~(new & (a > j))
+    base = None
+    for gap in (0, 5):
+        # physical layout: old | gap (NaN: never read) | new | y
+        Ap = np.full((n, p + gap + 1), np.nan)
+        Ap[:, :p_old] = A[:, :p_old]
+        Ap[:, p_old + gap:] = A[:, p_old:]
+        for cross in ((False, True) if p_old > 0 else (False,)):
+            rc, out, cover, st = emu.gram_plan(Ap, p_old, c, cap, warps, kchunks, mode, gap=gap, cross_only=cross,
+                                               allow_loose=loose, pad_mode=pad, force_r=force_r)
+            assert rc == 0, (gap, cross, rc)
+            want = needed & ~new if cross else needed
+            skipped = new if cross else new & (a // 8 > j // 8)        # whole 8 x 8 fragments below the diagonal
+            assert np.all(cover[want] == 1) and np.all(cover[skipped] == 0) and np.all(cover <= 1), (gap, cross)
+            assert np.allclose(out[want], ref[want], rtol=1e-12, atol=1e-12)
+            assert st['max_slots'] <= cap and st['max_positions_per_tile'] <= 4 * warps
+            assert st['max_runs'] <= st['max_slots'] // 2
+            assert 1 <= st['min_ksplit'] <= st['max_ksplit'] <= (min(force_r, kchunks) if force_r else kchunks)
+            if not loose:
+                assert st['loose'] == 0 and st['max_ksplit'] == 1
+            if pad >= 0 and ((c + 7) // 8) % 2 == 1:
+                assert st['pad'] == pad
+            if not cross:
+                if gap == 0:
+                    base = (out, st)
+                else:
+                    # the same plan on physical columns: the same logical block, bit for bit
+                    assert np.array_equal(out, base[0], equal_nan=True)
+                    assert {k: v for k, v in st.items()} == base[1]
+
+
+def test_gram_plan_reaches_every_kernel_form():
+    """The forms the GPU reference tests name (tests/test_gpu_gram_ref.py) exist in the plans of their shapes: the
+    all-loose warp form FLEX 2 (p_old = 1, c = 146 at 15 warps; 400 + 17 at 12), a k-split, both pad layouts, every
+    box kind and multi-tile plans (the 352-slot cap)."""
+    def st(p_old, c, warps=15, kchunks=1, **kw):
+        rc, _, _, s = emu.gram_plan(None, p_old, c, 352, warps, kchunks, 2, **kw)
+        assert rc == 0
+        return s
+    assert st(1, 146)['flex2'] > 0 and st(400, 17, warps=12)['flex2'] > 0
+    assert st(28, 168)['flex2'] == 0 and st(28, 168)['flex0'] > 0 and st(28, 168)['flex1'] > 0
+    assert st(50, 8, kchunks=4)['max_ksplit'] == 4 and st(58, 168)['max_ksplit'] == 1
+    assert st(8, 17)['pad'] == 1 and st(16, 33)['pad'] == 0
+    s = st(20, 300)
+    assert s['box8'] > 0 and s['box32'] > 0 and s['box128'] > 0 and s['n_tiles'] > 1
+    assert st(400, 1680)['n_tiles'] == 168
+    # the cp.async plan of a wide tile: masked 2 x 2 blocks, no loose ones
+    s = st(1, 146, warps=16, allow_loose=False)
+    assert s['loose'] == 0 and s['flex1'] + s['flex2'] > 0
+
+
 @pytest.mark.parametrize('e', [0, 1, 2])
 def test_derivative_factor_math_matches_oracle(cubic_table, phis_cubic, bern_table, phis_bern, e):
     """The device's bss_derivatives factor math (fokl_math.cuh: twice_normalised, cubic_basis_d1/d2,
