@@ -55,6 +55,14 @@ B200_CONFIG = {
 _ENGINES = {}
 LAST_FIT_INFO = {}
 
+# evaluate / coverage3 / bss_derivatives reduce the N x draws product on the device (fokl_predict_summary: mean and two
+# order statistics per row, the same bits as numpy on the full product) once it has at least this many cells; smaller
+# products are copied to the host and reduced by numpy (fokl_predict_draws)
+_PREDICT_SUMMARY_MIN_CELLS = 1 << 24
+# rows of the design matrix built per K1 launch on the summary path (a multiple of 16 for K1's 16-byte stores): bounds
+# the device memory of a prediction independently of N
+_PREDICT_CHUNK_ROWS = 1 << 16
+
 
 def _engine(device=None):
     """One Engine (CUDA context handle + scratch) per (process, device)."""
@@ -535,7 +543,8 @@ class FoKL:
                 warnings.warn("Cleaning was already performed on default 'inputs', so overriding 'clean' to False.",
                               category=UserWarning)
                 current['clean'] = False
-            normputs = self.inputs
+            resident = self._resident_inputs()
+            normputs = resident if resident is not None else self.inputs
         elif current['clean']:
             normputs = self.clean(inputs, kwargs_from_other=kwargs_to_clean)
         else:
@@ -543,10 +552,13 @@ class FoKL:
 
         betas = np.asarray(betas, dtype=np.float64)
         m, mbets = np.shape(betas)
-        normputs = np.asarray(normputs, dtype=np.float64)
-        n = np.shape(normputs)[0]
-        mputs = int(np.size(normputs) / n)
-        normputs = normputs.reshape(n, mputs)
+        if isinstance(normputs, _DeviceInputs):
+            n, mputs = normputs.ds.n, normputs.ds.m
+        else:
+            normputs = np.asarray(normputs, dtype=np.float64)
+            n = np.shape(normputs)[0]
+            mputs = int(np.size(normputs) / n)
+            normputs = normputs.reshape(n, mputs)
 
         if self.setnos is None:
             setnos = np.random.choice(m, draws, replace=False)
@@ -558,7 +570,21 @@ class FoKL:
 
         terms = np.asarray(mtx, dtype=np.float64).reshape(mbets - 1, mputs) if mbets > 1 else np.zeros((0, mputs))
         eng = _engine()
-        modells = eng_predict(eng, self.phis, self.kernel, normputs, terms, betas[np.asarray(setnos)[:draws], :])
+        betas_sel = betas[np.asarray(setnos)[:draws], :]
+        if draws >= 2 and betas_sel.shape[0] == draws and n * draws >= _PREDICT_SUMMARY_MIN_CELLS:
+            cut = int(np.floor(draws * 0.025) + 1)
+            with_bounds = current['ReturnBounds'] == True  # noqa: E712
+            mean, lo, hi = eng_predict_summary(eng, self.phis, self.kernel, normputs, terms, betas_sel,
+                                               (cut, draws - cut) if with_bounds else None)
+            if with_bounds:
+                bounds = np.zeros((n, 2))
+                bounds[:, 0] = lo
+                bounds[:, 1] = hi
+                return mean, bounds
+            return mean
+        if isinstance(normputs, _DeviceInputs):
+            normputs = self.inputs
+        modells = eng_predict(eng, self.phis, self.kernel, normputs, terms, betas_sel)
         mean = np.mean(modells, 1)
 
         if current['ReturnBounds'] == True:  # noqa: E712  (reference semantics: 1 == True)
@@ -569,6 +595,14 @@ class FoKL:
             bounds[:, 1] = srt[:, draws - cut]
             return mean, bounds
         return mean
+
+    def _resident_inputs(self):
+        """The default inputs when they live only in HBM (fit(clean=True) on a large dataset) and this process is the only
+        rank, so evaluate may read them there; None otherwise."""
+        v = self.__dict__.get('inputs')
+        if isinstance(v, _DeviceInputs) and _engine().world == 1:
+            return v
+        return None
 
     def coverage3(self, **kwargs):
         """Validation: predicted mean, confidence bounds and 'rmse' over a dataset (FR:982-1200).
@@ -596,6 +630,8 @@ class FoKL:
             current['plot'] = _str_to_bool(current['plot'])
         for boolean in ['bounds', 'labels', 'legend']:
             current[boolean] = _str_to_bool(current[boolean])
+        # device-resident default inputs: evaluate(None) reads them in HBM; the plot materialises them only for `xaxis`
+        resident = current['inputs'] is None and self._resident_inputs() is not None
 
         warn_plot = ' and ignoring plot.' if current['plot'] else '.'
         for this, other in (('inputs', 'data'), ('data', 'inputs')):
@@ -608,7 +644,7 @@ class FoKL:
                           "Returning a regular plot instead.", category=UserWarning)
             current['plot'] = True
 
-        if current['inputs'] is None:
+        if current['inputs'] is None and not resident:
             current['inputs'] = self.inputs
         if current['data'] is None:
             current['data'] = self.data
@@ -628,6 +664,8 @@ class FoKL:
                                  _suppress_normalization_warning=True)
 
         if current['plot']:
+            if resident and current['xaxis'] is not False and isinstance(current['xaxis'], int):
+                normputs = self.inputs
             self._plot_coverage(current, normputs, data, mean, bounds)
 
         if data is not False:
@@ -645,7 +683,7 @@ class FoKL:
         except ImportError:
             warnings.warn("matplotlib is not installed; skipping the coverage3 plot.", category=UserWarning)
             return
-        n = np.shape(normputs)[0]
+        n = len(mean)
         if current['xaxis'] is False:
             plt_x = np.linspace(0, n - 1, n)
         elif isinstance(current['xaxis'], int):
@@ -980,7 +1018,9 @@ class FoKL:
                     dr = np.zeros((len(idx), M), dtype=np.uint8)
                     dr[:, m] = di + 1
                     d_rows.append(dr)
-        dy = np.zeros([N, M, 2, draws])
+        # the mean over the draws on the device, without the N x M x 2 x draws array (same bits as np.mean on axis 3)
+        mean_only = not current['IndividualDraws'] and draws > 1 and N * draws >= _PREDICT_SUMMARY_MIN_CELLS
+        dy = np.zeros([N, M, 2, 1 if mean_only else draws])
         bsel = np.ascontiguousarray(betas[-draws:, :], dtype=np.float64)
         if t_rows and bsel.shape[0] != draws:
             # upstream fails here as well: `betas[-draws:, b + 1] * phi` does not broadcast into dy's draws axis (FR:789)
@@ -988,9 +1028,9 @@ class FoKL:
                              f"'betas' holds fewer than draws={draws} rows.")
         if t_rows:
             eng_derivative_draws(_engine(), phis, kernel, inputs, np.concatenate(t_rows, axis=0),
-                                 np.concatenate(d_rows, axis=0), divisors, pairs, bsel, dy)
+                                 np.concatenate(d_rows, axis=0), divisors, pairs, bsel, dy, mean_only)
 
-        if not current['IndividualDraws'] and draws > 1:
+        if not current['IndividualDraws'] and draws > 1 and not mean_only:
             dy = np.mean(dy, axis=3)[:, :, :, np.newaxis]
         if not current['ReturnFullArray']:
             dy = np.concatenate([dy[:, :, 0, :], dy[:, :, 1, :]], axis=1)
@@ -1066,12 +1106,13 @@ class FoKL:
         return filepath
 
 
-def eng_derivative_draws(eng, phis, kernel, inputs, term_rows, deriv_rows, divisors, pairs, bsel, dy):
+def eng_derivative_draws(eng, phis, kernel, inputs, term_rows, deriv_rows, divisors, pairs, bsel, dy, mean_only=False):
     """dy[:, m, di, :] = (derivative design columns of the terms idx that contain input m) @ bsel[:, idx + 1]' for every
     (m, di, idx, off) of `pairs`, on the device: one fokl_basis_build_deriv over all rows of term_rows / deriv_rows (the
-    columns of a pair start at row `off`), one fokl_predict_draws per pair (FR:727-795)."""
+    columns of a pair start at row `off`), one fokl_predict_draws per pair (FR:727-795).  mean_only: dy[:, m, di, 0] =
+    the mean over the draws instead, from fokl_predict_summary."""
     import torch
-    N, M, draws = np.shape(inputs)[0], np.shape(term_rows)[1], dy.shape[3]
+    N, M, draws = np.shape(inputs)[0], np.shape(term_rows)[1], bsel.shape[0]
     eng.set_phis(phis, kernel)
     x64 = np.ascontiguousarray(inputs, dtype=np.float64)
     ds = eng.upload(x64, np.zeros(N))
@@ -1087,6 +1128,12 @@ def eng_derivative_draws(eng, phis, kernel, inputs, term_rows, deriv_rows, divis
         if not len(idx):
             continue
         b = torch.from_numpy(np.ascontiguousarray(bsel[:, idx + 1])).to(eng.device)
+        if mean_only:
+            mean = torch.empty((N,), dtype=torch.float64, device=eng.device)
+            eng._ck(eng.lib.fokl_predict_summary(eng.ctx, X[off].data_ptr(), ds.ldx, N, len(idx), b.data_ptr(), draws,
+                                                 -1, -1, mean.data_ptr(), None, None))
+            dy[:, m, di, 0] = mean.cpu().numpy()
+            continue
         out = torch.empty((N, draws), dtype=torch.float64, device=eng.device)
         eng._ck(eng.lib.fokl_predict_draws(eng.ctx, X[off].data_ptr(), ds.ldx, N, len(idx), b.data_ptr(), draws,
                                            out.data_ptr()))
@@ -1111,3 +1158,38 @@ def eng_predict(eng, phis, kernel, normputs, terms, betas_sel):
     eng._ck(eng.lib.fokl_predict_draws(eng.ctx, X.data_ptr(), ds.ldx, n, p, b.data_ptr(), b.shape[0], out.data_ptr()))
     eng.synchronize()
     return out.cpu().numpy()
+
+
+def eng_predict_summary(eng, phis, kernel, normputs_or_ds, terms, betas_sel, ranks):
+    """Per row i of X(normputs) @ betas_sel': (mean over the draws, value at ascending rank ranks[0], at ranks[1]), the
+    bits of np.mean(modells, 1) and np.sort(modells, 1)[:, k] (only the sign of a zero may differ); the last two are
+    None when `ranks` is None.  normputs_or_ds is a host array or device-resident _DeviceInputs.  The design matrix is
+    built _PREDICT_CHUNK_ROWS rows at a time and the product is reduced on the device, so device memory does not grow
+    with N beyond the inputs and the three output columns."""
+    import torch
+    eng.set_phis(phis, kernel)
+    if isinstance(normputs_or_ds, _DeviceInputs):
+        ds = normputs_or_ds.ds
+    else:
+        ds = eng.upload(normputs_or_ds, np.zeros(normputs_or_ds.shape[0]))
+    n, p = ds.n, terms.shape[0] + 1
+    b = torch.from_numpy(np.ascontiguousarray(betas_sel, dtype=np.float64)).to(eng.device)
+    rank_lo, rank_hi = ranks if ranks is not None else (-1, -1)
+    out = torch.empty((1 if ranks is None else 3, n), dtype=torch.float64, device=eng.device)
+    rows = min(_PREDICT_CHUNK_ROWS, (n + 15) // 16 * 16)
+    X = torch.empty((p, rows), dtype=torch.float64, device=eng.device)
+    eng._ck(eng.lib.fokl_fill_ones(eng.ctx, X.data_ptr(), rows))
+    t16 = np.ascontiguousarray(terms, dtype=np.int16)
+    for r0 in range(0, n, rows):
+        nr = min(rows, n - r0)
+        if p > 1:
+            eng._ck(eng.lib.fokl_basis_build(eng.ctx, eng.kernel_id, ds.x.data_ptr() + 8 * r0, nr, ds.ldx, ds.m,
+                                             t16.ctypes.data, p - 1, X[1].data_ptr(), rows))
+        lo_ptr, hi_ptr = (None, None) if ranks is None else (out[1].data_ptr() + 8 * r0, out[2].data_ptr() + 8 * r0)
+        eng._ck(eng.lib.fokl_predict_summary(eng.ctx, X.data_ptr(), rows, nr, p, b.data_ptr(), b.shape[0], rank_lo,
+                                             rank_hi, out[0].data_ptr() + 8 * r0, lo_ptr, hi_ptr))
+    eng.synchronize()
+    res = out.cpu().numpy()
+    if ranks is None:
+        return res[0], None, None
+    return res[0], res[1], res[2]

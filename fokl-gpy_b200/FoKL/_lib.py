@@ -11,8 +11,8 @@ CSRC = os.path.join(os.path.dirname(_HERE), 'csrc')
 SO_PATH = os.path.join(CSRC, 'libfokl_b200.so')
 if os.environ.get('FOKL_B200_LIB'):        # kernel-variant experiments (tools/): another build of the same sources
     SO_PATH = os.path.abspath(os.environ['FOKL_B200_LIB'])
-SOURCES = ['ctx.cu', 'basis.cu', 'gram.cu', 'candidates.cu', 'nested.cu', 'update.cu']
-HEADERS = ['fokl_ctx.cuh', 'fokl_math.cuh', 'cand_math.cuh', 'gram_plan.h', 'eigbig.cuh', 'killbig.cuh', 'update_math.cuh']
+SOURCES = ['ctx.cu', 'basis.cu', 'gram.cu', 'candidates.cu', 'nested.cu', 'update.cu', 'predict.cu']
+HEADERS = ['fokl_ctx.cuh', 'fokl_math.cuh', 'cand_math.cuh', 'gram_plan.h', 'eigbig.cuh', 'killbig.cuh', 'update_math.cuh', 'predict_math.cuh']
 
 ABI_VERSION = 2
 KERNEL_CUBIC, KERNEL_BERNOULLI = 0, 1
@@ -84,6 +84,7 @@ PROTOTYPES = {
                               ctypes.POINTER(KillParams), _vp, _vp]),
     'fokl_residual_moments': (_i32, [_vp, _vp, _i64, _i64, _i32, _vp, _vp, _vp, _vp]),
     'fokl_predict_draws': (_i32, [_vp, _vp, _i64, _i64, _i32, _vp, _i32, _vp]),
+    'fokl_predict_summary': (_i32, [_vp, _vp, _i64, _i64, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _vp]),
     'fokl_column_minmax': (_i32, [_vp, _vp, _i64, _i64, _i32, _vp]),
     'fokl_normalize': (_i32, [_vp, _vp, _i64, _i64, _i32, _vp]),
 }

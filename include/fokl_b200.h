@@ -273,6 +273,14 @@ int fokl_residual_moments(fokl_ctx *ctx, const double *X, int64_t ld, int64_t n,
 int fokl_predict_draws(fokl_ctx *ctx, const double *X, int64_t ld, int64_t n, int p, const double *betas,
                        int n_draws, double *out);
 
+/* evaluate at training-set scale: with v[i][d] = sum_j X[i][j] * betas[d][j] (the bits of fokl_predict_draws),
+ * mean_out[i] = np.mean(v[i]) and, unless rank_lo = rank_hi = -1 (mean only; lo_out / hi_out may be NULL),
+ * lo_out[i] / hi_out[i] = np.sort(v[i])[rank_lo / rank_hi], bit for bit (NaN sorts last; only the sign of a zero may
+ * differ).  X column-major (ld), betas row-major n_draws x p, outputs n doubles each (all dev).  The product is
+ * formed in L2-sized row chunks and never written out: device scratch depends on n_draws, not on n. */
+int fokl_predict_summary(fokl_ctx *ctx, const double *X, int64_t ld, int64_t n, int p, const double *betas,
+                         int n_draws, int rank_lo, int rank_hi, double *mean_out, double *lo_out, double *hi_out);
+
 /* clean/_normalize on device (FR:377, 436-437): minmax_out (dev, 2*m) = per-column min, max of x
  * (column-major n x m, ldx); then fokl_normalize applies x = (x - min) / (max - min) in place with
  * minmax (host, 2*m). */
