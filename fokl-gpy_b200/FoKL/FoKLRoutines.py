@@ -62,6 +62,13 @@ _PREDICT_SUMMARY_MIN_CELLS = 1 << 24
 # rows of the design matrix built per K1 launch on the summary path (a multiple of 16 for K1's 16-byte stores): bounds
 # the device memory of a prediction independently of N
 _PREDICT_CHUNK_ROWS = 1 << 16
+# bss_derivatives streams its rows through fokl_deriv_summary (eng_derivative_summary) once N * draws reaches this many
+# cells and draws > 1 -- evaluate's rule.  It is a name of its own so that the mean-only path through
+# fokl_predict_summary (eng_derivative_draws) stays selectable on its own.
+_DERIV_SUMMARY_MIN_CELLS = 1 << 24
+# device bytes of one row chunk of dy on that path (N x M x 2 x draws with IndividualDraws=True): fewer rows per chunk
+# than _PREDICT_CHUNK_ROWS when a chunk would be larger
+_DERIV_CHUNK_BYTES = 256 << 20
 
 
 def _engine(device=None):
@@ -669,8 +676,14 @@ class FoKL:
             self._plot_coverage(current, normputs, data, mean, bounds)
 
         if data is not False:
-            # reference quirk kept (FR:1193): (n,) - (n, 1) broadcasts to n x n; equals |mean(mean) - mean(data)|
-            rmse = np.sqrt(np.mean(mean - data) ** 2)
+            d = np.asarray(data)
+            if d.ndim == 2 and d.shape[1] == 1 and np.size(mean) * d.shape[0] > _PREDICT_SUMMARY_MIN_CELLS:
+                # the reference's expression (FR:1193) broadcasts (n,) - (n, 1) to an n x n array; the mean of
+                # mean_c - data_r over all (r, c) is mean(mean) - mean(data), equal up to the last bits
+                rmse = np.abs(np.mean(mean) - np.mean(d))
+            else:
+                # reference quirk kept (FR:1193): (n,) - (n, 1) broadcasts to n x n; equals |mean(mean) - mean(data)|
+                rmse = np.sqrt(np.mean(mean - data) ** 2)
         else:
             rmse = []
         if current['ReturnBounds'] == True:  # noqa: E712
@@ -921,23 +934,23 @@ class FoKL:
         """Gradient (or chosen first / second partial derivatives) of the fitted function with respect to the inputs
         (FR:594-805).  Keywords as upstream: inputs, kernel, d1, d2, draws, betas, phis, mtx, minmax, IndividualDraws,
         ReturnFullArray, ReturnBasis.  The derivative design matrices come from the derivative form of the basis
-        kernel (fokl_basis_build_deriv) and the products with the draws from fokl_predict_draws, both on the device."""
+        kernel (fokl_basis_build_deriv) and the products with the draws from fokl_predict_draws, both on the device.
+        Once N * draws >= _DERIV_SUMMARY_MIN_CELLS (draws > 1) the rows stream through fokl_deriv_summary in chunks
+        instead (same bits), and device-resident default inputs (fit(clean=True)) are read in place."""
         default = {'inputs': None, 'kernel': self.kernel, 'd1': None, 'd2': None, 'draws': self.draws, 'betas': None,
                    'phis': None, 'mtx': self.mtx, 'minmax': self.minmax, 'IndividualDraws': False,
                    'ReturnFullArray': False, 'ReturnBasis': False}
         current = _process_kwargs(default, kwargs)
         for boolean in ['IndividualDraws', 'ReturnFullArray', 'ReturnBasis']:
             current[boolean] = _str_to_bool(current[boolean])
-        inputs = self.inputs if current['inputs'] is None else current['inputs']
+        resident = self._resident_inputs() if current['inputs'] is None else None
+        inputs = resident if resident is not None else (self.inputs if current['inputs'] is None else current['inputs'])
         betas = self.betas if current['betas'] is None else current['betas']
         phis = self.phis if current['phis'] is None else current['phis']
         kernel, draws, span = current['kernel'], current['draws'], current['minmax']
         if isinstance(kernel, int):
             kernel = self.kernels[kernel]
 
-        inputs = np.array(inputs)
-        if inputs.ndim == 1:
-            inputs = inputs[:, np.newaxis]
         if isinstance(betas, list):
             betas = np.array(betas)
             if betas.ndim == 1:
@@ -951,10 +964,23 @@ class FoKL:
                 mtx = mtx[:, np.newaxis]
         if len(span) == 2 and not isinstance(span[0], (list, np.ndarray)):
             span = [span]
-        if np.max(np.max(inputs)) > 1 or np.min(np.min(inputs)) < 0:
+        if resident is not None and not (draws > 1 and resident.ds.n * draws >= _DERIV_SUMMARY_MIN_CELLS
+                                         and resident.ds.m == np.shape(mtx)[1] and not current['ReturnBasis']):
+            resident, inputs = None, self.inputs        # a path that reads the inputs on the host
+        if resident is None:
+            inputs = np.array(inputs)
+            if inputs.ndim == 1:
+                inputs = inputs[:, np.newaxis]
+        if resident is not None:
+            xr = resident.ds.x[:, :resident.ds.n]
+            outside = bool(xr.max() > 1) or bool(xr.min() < 0)
+            N = resident.ds.n
+        else:
+            outside = np.max(np.max(inputs)) > 1 or np.min(np.min(inputs)) < 0
+            N = np.shape(inputs)[0]
+        if outside:
             warnings.warn("Input 'inputs' should be normalized (0-1). Auto-normalization is in-development.",
                           category=UserWarning)
-        N = np.shape(inputs)[0]
         B, M = np.shape(mtx)
         betas = np.asarray(betas, dtype=np.float64)
         if B != np.shape(betas)[1] - 1:
@@ -1018,15 +1044,21 @@ class FoKL:
                     dr = np.zeros((len(idx), M), dtype=np.uint8)
                     dr[:, m] = di + 1
                     d_rows.append(dr)
+        # the rows in chunks through fokl_deriv_summary, which also averages over the draws unless IndividualDraws
+        streamed = draws > 1 and N * draws >= _DERIV_SUMMARY_MIN_CELLS
         # the mean over the draws on the device, without the N x M x 2 x draws array (same bits as np.mean on axis 3)
-        mean_only = not current['IndividualDraws'] and draws > 1 and N * draws >= _PREDICT_SUMMARY_MIN_CELLS
+        mean_only = not current['IndividualDraws'] and draws > 1 and (
+            streamed or N * draws >= _PREDICT_SUMMARY_MIN_CELLS)
         dy = np.zeros([N, M, 2, 1 if mean_only else draws])
         bsel = np.ascontiguousarray(betas[-draws:, :], dtype=np.float64)
         if t_rows and bsel.shape[0] != draws:
             # upstream fails here as well: `betas[-draws:, b + 1] * phi` does not broadcast into dy's draws axis (FR:789)
             raise ValueError(f"operands could not be broadcast together with shapes ({draws},) ({bsel.shape[0]},): "
                              f"'betas' holds fewer than draws={draws} rows.")
-        if t_rows:
+        if t_rows and streamed:
+            eng_derivative_summary(_engine(), phis, kernel, inputs, np.concatenate(t_rows, axis=0),
+                                   np.concatenate(d_rows, axis=0), divisors, pairs, bsel, dy)
+        elif t_rows:
             eng_derivative_draws(_engine(), phis, kernel, inputs, np.concatenate(t_rows, axis=0),
                                  np.concatenate(d_rows, axis=0), divisors, pairs, bsel, dy, mean_only)
 
@@ -1138,6 +1170,66 @@ def eng_derivative_draws(eng, phis, kernel, inputs, term_rows, deriv_rows, divis
         eng._ck(eng.lib.fokl_predict_draws(eng.ctx, X[off].data_ptr(), ds.ldx, N, len(idx), b.data_ptr(), draws,
                                            out.data_ptr()))
         dy[:, m, di, :] = out.cpu().numpy()
+
+
+def eng_derivative_summary(eng, phis, kernel, inputs, term_rows, deriv_rows, divisors, pairs, bsel, dy):
+    """dy as eng_derivative_draws fills it -- the same bits -- with the rows streamed through fokl_deriv_summary: per
+    chunk one call builds the chunk's derivative columns and forms every pair's values (dy of shape (N, M, 2, draws)) or
+    their mean over the draws (dy of shape (N, M, 2, 1)), in dy's layout on the device; one copy per chunk brings the
+    slice dy[r0:r0 + rows] back.  inputs is a host array or device-resident _DeviceInputs.  Device memory: the inputs,
+    the betas blocks, one chunk of dy (at most _DERIV_CHUNK_BYTES) and the library's chunk workspace."""
+    import torch
+    N, M, _, depth = dy.shape
+    draws = bsel.shape[0]
+    eng.set_phis(phis, kernel)
+    if isinstance(inputs, _DeviceInputs):
+        ds = inputs.ds
+    else:
+        ds = eng.upload(np.ascontiguousarray(inputs, dtype=np.float64), np.zeros(N))
+    t16 = np.ascontiguousarray(term_rows, dtype=np.int16)
+    d8 = np.ascontiguousarray(deriv_rows, dtype=np.uint8)
+    dv = np.ascontiguousarray(divisors, dtype=np.float64)
+    table, blocks, boff = [], [], 0
+    for m, di, idx, off in pairs:
+        table.append((off, len(idx), boff, m, di))
+        blocks.append(np.ascontiguousarray(bsel[:, idx + 1]).ravel())
+        boff += draws * len(idx)
+    table = np.ascontiguousarray(table, dtype=np.int64)
+    b = torch.from_numpy(np.concatenate(blocks)).to(eng.device)
+    per_row = M * 2 * depth
+    rows = max(16, min(_PREDICT_CHUNK_ROWS, _DERIV_CHUNK_BYTES // (8 * per_row)) // 16 * 16)
+    rows = min(rows, (N + 15) // 16 * 16)
+    out = torch.empty((rows * per_row,), dtype=torch.float64, device=eng.device)
+    cuda = out.device.type == 'cuda'
+    # two pinned buffers: the host copies chunk k - 1 into dy while the device works on chunk k
+    host = [torch.empty((rows * per_row,), dtype=torch.float64, pin_memory=cuda) for _ in range(2)]
+    pending = [None, None]
+    flat = dy.reshape(N, per_row)
+
+    def drain(s):
+        if pending[s] is not None:
+            r0, nr, done = pending[s]
+            if done is not None:
+                done.synchronize()
+            flat[r0:r0 + nr] = host[s][:nr * per_row].numpy().reshape(nr, per_row)
+            pending[s] = None
+
+    for k, r0 in enumerate(range(0, N, rows)):
+        nr, s = min(rows, N - r0), k % 2
+        drain(s)
+        eng._ck(eng.lib.fokl_deriv_summary(eng.ctx, eng.kernel_id, ds.x.data_ptr(), ds.ldx, M, r0, nr,
+                                           t16.ctypes.data, d8.ctypes.data, dv.ctypes.data, t16.shape[0],
+                                           table.ctypes.data, len(table), b.data_ptr(), draws,
+                                           1 if depth == 1 else 0, out.data_ptr()))
+        host[s][:nr * per_row].copy_(out[:nr * per_row], non_blocking=cuda)
+        done = None
+        if cuda:
+            done = torch.cuda.Event()
+            done.record()
+        pending[s] = (r0, nr, done)
+    eng.synchronize()       # surfaces the out-of-range flag (inputs outside [0, 1]) as ValueError
+    drain(0)
+    drain(1)
 
 
 def eng_predict(eng, phis, kernel, normputs, terms, betas_sel):

@@ -85,6 +85,8 @@ PROTOTYPES = {
     'fokl_residual_moments': (_i32, [_vp, _vp, _i64, _i64, _i32, _vp, _vp, _vp, _vp]),
     'fokl_predict_draws': (_i32, [_vp, _vp, _i64, _i64, _i32, _vp, _i32, _vp]),
     'fokl_predict_summary': (_i32, [_vp, _vp, _i64, _i64, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _vp]),
+    'fokl_deriv_summary': (_i32, [_vp, _i32, _vp, _i64, _i32, _i64, _i64, _vp, _vp, _vp, _i32, _vp, _i32, _vp, _i32,
+                                  _i32, _vp]),
     'fokl_column_minmax': (_i32, [_vp, _vp, _i64, _i64, _i32, _vp]),
     'fokl_normalize': (_i32, [_vp, _vp, _i64, _i64, _i32, _vp]),
 }

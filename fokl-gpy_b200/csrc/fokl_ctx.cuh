@@ -53,7 +53,7 @@ struct fokl_ctx {
     bool ev_eig_set = false;
 
     // growable scratch buffers, indexed by purpose
-    enum { B_META = 0, B_BASIS, B_GRAM, B_CAND_A, B_CAND_B, B_CAND_C, B_CAND_D, B_MISC, B_PREDICT, B_COUNT };
+    enum { B_META = 0, B_BASIS, B_GRAM, B_CAND_A, B_CAND_B, B_CAND_C, B_CAND_D, B_MISC, B_PREDICT, B_DERIV, B_COUNT };
     fokl_buf bufs[B_COUNT];
 };
 

@@ -281,6 +281,22 @@ int fokl_predict_draws(fokl_ctx *ctx, const double *X, int64_t ld, int64_t n, in
 int fokl_predict_summary(fokl_ctx *ctx, const double *X, int64_t ld, int64_t n, int p, const double *betas,
                          int n_draws, int rank_lo, int rank_hi, double *mean_out, double *lo_out, double *hi_out);
 
+/* bss_derivatives at training-set scale, one row chunk: rows [r0, r0 + rows) of x (dev, column-major, ldx, m inputs).
+ * terms / deriv / divisors / c as fokl_basis_build_deriv (host); the chunk's c derivative columns are built with its
+ * kernels into device scratch.  pairs (host, n_pairs x 5 int64): {column offset, width, betas offset, input, order - 1};
+ * pair k's betas block is betas[offset .. + n_draws * width) (dev, row-major n_draws x width) and its values are
+ * v[i][d] = sum_j W[i][offset + j] * b[d][j] with the FMA order of fokl_predict_draws (the same bits).  out (dev) gets
+ * the C-order slice dy[r0 : r0 + rows] of bss_derivatives' dy: mean_only = 0: [rows][m][2][n_draws] of v;
+ * mean_only = 1: [rows][m][2] of np.mean(v[i]) over the draws (the bits of fokl_predict_summary).  (input, order)
+ * slots no pair names, and pairs of width 0, get 0.0.  Device scratch: 8 * c * rows bytes, plus (mean_only) at most
+ * 32 MB of values; it does not depend on the rows outside the chunk.  A bad pointer, column range, betas offset, input,
+ * order, repeated slot, n_draws or term list returns FOKL_EINVAL before anything is written to out; inputs outside
+ * [0, 1] set the deferred FOKL_ERANGE flag (cubic). */
+int fokl_deriv_summary(fokl_ctx *ctx, int kernel, const double *x, int64_t ldx, int m, int64_t r0, int64_t rows,
+                       const int16_t *terms, const uint8_t *deriv, const double *divisors, int c,
+                       const int64_t *pairs, int n_pairs, const double *betas, int n_draws, int mean_only,
+                       double *out);
+
 /* clean/_normalize on device (FR:377, 436-437): minmax_out (dev, 2*m) = per-column min, max of x
  * (column-major n x m, ldx); then fokl_normalize applies x = (x - min) / (max - min) in place with
  * minmax (host, 2*m). */
