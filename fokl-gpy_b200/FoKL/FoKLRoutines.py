@@ -69,6 +69,9 @@ _DERIV_SUMMARY_MIN_CELLS = 1 << 24
 # device bytes of one row chunk of dy on that path (N x M x 2 x draws with IndividualDraws=True): fewer rows per chunk
 # than _PREDICT_CHUNK_ROWS when a chunk would be larger
 _DERIV_CHUNK_BYTES = 256 << 20
+# `clean` (fit(clean=True), evaluate(inputs, clean=True)) formats, normalises and splits the dataset in HBM once the raw
+# inputs have at least this many cells; smaller datasets take the host path, where the pass over them costs little
+_CLEAN_ON_DEVICE_MIN_CELLS = 1 << 20
 
 
 def _engine(device=None):
@@ -263,8 +266,9 @@ class FoKL:
     # ------------------------------------------------------------------------------------------------
     # dataset formatting (host side; FR:248-542)
     # ------------------------------------------------------------------------------------------------
-    def _format(self, inputs, data=None, AutoTranspose=True, SingleInstance=False, bit=64, _copy=True):
-        """inputs -> [n x m] ndarray, data -> [n x 1] ndarray (FR:248-316)."""
+    def _format(self, inputs, data=None, AutoTranspose=True, SingleInstance=False, bit=64, _copy=True, _widen=True):
+        """inputs -> [n x m] ndarray, data -> [n x 1] ndarray (FR:248-316).  _widen=False: float32 inputs are returned
+        as float32 (with the same warning) for the caller to widen on the device, where the conversion is exact too."""
         import pandas as pd
         AutoTranspose = _str_to_bool(AutoTranspose)
         SingleInstance = _str_to_bool(SingleInstance)
@@ -290,7 +294,8 @@ class FoKL:
         if inputs.ndim > 2:
             inputs = np.squeeze(inputs)
         if inputs.dtype != datatype:
-            inputs = np.array(inputs, dtype=datatype)
+            if _widen or not (inputs.dtype == np.float32 and datatype == np.float64):
+                inputs = np.array(inputs, dtype=datatype)
             warnings.warn(f"'inputs' was converted to float{bit}. May require user-confirmation that "
                           f"values did not get corrupted.", category=UserWarning)
         if inputs.ndim == 1:
@@ -553,7 +558,7 @@ class FoKL:
             resident = self._resident_inputs()
             normputs = resident if resident is not None else self.inputs
         elif current['clean']:
-            normputs = self.clean(inputs, kwargs_from_other=kwargs_to_clean)
+            normputs = self._evaluate_clean(inputs, kwargs_to_clean, draws)
         else:
             normputs = np.array(inputs)
 
@@ -590,7 +595,7 @@ class FoKL:
                 return mean, bounds
             return mean
         if isinstance(normputs, _DeviceInputs):
-            normputs = self.inputs
+            normputs = self.inputs if normputs is self.__dict__.get('inputs') else normputs.to_numpy()
         modells = eng_predict(eng, self.phis, self.kernel, normputs, terms, betas_sel)
         mean = np.mean(modells, 1)
 
@@ -727,36 +732,82 @@ class FoKL:
             plt.legend()
         plt.show()
 
-    def _clean_on_device(self, inputs, data, kwargs_to_clean):
-        """`clean` for `fit(clean=True)` with the normalisation (FR:373-377, 436-437) done in HBM: the raw inputs are
-        copied to the device once, per-column min / max and (x - min) / (max - min) run there (bit-identical to the
-        host expression), and `self.inputs` is materialised on the host only if somebody reads it.  Returns the
-        DeviceDataset, or None when the request needs the host path (train < 1, bit != 64, normalize=False, more
-        than 32 inputs, small datasets where the host pass is free)."""
-        current = _process_kwargs(dict(_CLEAN_DEFAULTS), dict(kwargs_to_clean))
-        if current['train'] != 1 or current['bit'] != 64 or _str_to_bool(current['normalize']) is not True:
+    def _device_raw_inputs(self, inputs, current):
+        """The raw `inputs` of a `clean` request (keywords resolved in `current`) that may be formatted and normalised in
+        HBM without a host pass over them: float32 / float64 numpy arrays, and pandas frames of one such dtype (their
+        block goes up as it is), of at least _CLEAN_ON_DEVICE_MIN_CELLS cells, with bit=64 and normalize=True.  None
+        for anything else (mixed-dtype or object frames, other dtypes, small datasets): that takes the host path."""
+        if current['bit'] != 64 or _str_to_bool(current['normalize']) is not True:
             return None
+        floats = (np.dtype(np.float32), np.dtype(np.float64))
         try:
             import pandas as pd
-            if isinstance(inputs, (pd.DataFrame, pd.Series)) or isinstance(data, (pd.DataFrame, pd.Series)):
+            if isinstance(inputs, pd.DataFrame):
+                dtypes = set(inputs.dtypes)
+                ok = len(dtypes) == 1 and dtypes.pop() in floats
+                return inputs if ok and inputs.size >= _CLEAN_ON_DEVICE_MIN_CELLS else None
+            if isinstance(inputs, pd.Series):
                 return None
         except ImportError:
             pass
         raw = np.asarray(inputs)
-        if raw.dtype != np.float64 or np.asarray(data).dtype != np.float64 or raw.size < (1 << 20):
+        if raw.dtype not in floats or raw.size < _CLEAN_ON_DEVICE_MIN_CELLS:
             return None
+        return raw
+
+    def _clean_on_device(self, inputs, data, kwargs_to_clean):
+        """`clean` for `fit(clean=True)` done in HBM (FR:248-542): `_format`'s checks and warnings run on the host
+        unchanged, but the raw inputs go to the device as they are (float32 widened, a column-major block transposed
+        there), the per-column min / max and (x - min) / (max - min) run there (bit-identical to the host expression),
+        and a train split (`generate_trainlog` on the host, unchanged) keeps its rows with fokl_rows_compact.  Sets
+        `inputs` (the train rows, materialised on the host only if somebody reads them), `data` (the train rows) and
+        `trainlog` as the host path's `fit` leaves them.  Returns (DeviceDataset of the train rows, moments_on_device)
+        or None when the request needs the host path (_device_raw_inputs).  moments_on_device: the b / btau defaults
+        come from the device's sum(y), sum(y^2) -- only for the float64 numpy, train == 1, <= 32 input datasets that
+        took this path before the other forms did; every other form keeps the host path's np.var / np.mean of the train
+        data, so that its fit stays bit-identical to the host path."""
+        current = _process_kwargs(dict(_CLEAN_DEFAULTS), dict(kwargs_to_clean))
+        raw = self._device_raw_inputs(inputs, current)
+        if raw is None:
+            return None
+        numpy_f64 = isinstance(raw, np.ndarray) and raw.dtype == np.float64 and not hasattr(data, 'to_numpy') \
+            and np.asarray(data).dtype == np.float64
         raw, data = self._format(raw, data, current['AutoTranspose'], current['SingleInstance'], current['bit'],
-                                 _copy=False)
+                                 _copy=False, _widen=False)
         n, mm = raw.shape
-        if mm > 32 or data.shape[0] != n:
+        if data.shape[0] != n:
             return None
         eng = _engine()
         ds = eng.upload_clean(raw, data, lambda column_minmax: self._normalize_bounds(
             mm, column_minmax, current['minmax'], current['pillow'], current['pillow_type']))
+        trainlog = self.generate_trainlog(current['train'], n)
+        if trainlog is not None:
+            ds = eng.rows_compact(ds, trainlog)
+            data = data[trainlog]
         self.__dict__['inputs'] = _DeviceInputs(ds)
         self.data = data
-        self.trainlog = None
-        return ds
+        self.trainlog = trainlog
+        return ds, numpy_f64 and mm <= 32 and trainlog is None
+
+    def _evaluate_clean(self, inputs, kwargs_to_clean, draws):
+        """`self.clean(inputs, ...)` for `evaluate(inputs, clean=True)` on a model that already has `inputs` (so clean
+        sets no attribute and draws no random number).  When the prediction will be reduced on the device
+        (fokl_predict_summary) the raw rows are normalised in HBM with the bounds `_normalize_bounds` resolves (same
+        warnings, same self.minmax update) and returned as _DeviceInputs; otherwise the formatted rows are normalised on
+        the host as `clean` does."""
+        current = _process_kwargs(dict(_CLEAN_DEFAULTS), dict(kwargs_to_clean))
+        raw = self._device_raw_inputs(inputs, current) if 'inputs' in self.__dict__ and draws >= 2 else None
+        if raw is None or _engine().world != 1:
+            return self.clean(inputs, kwargs_from_other=kwargs_to_clean)
+        raw, _ = self._format(raw, None, current['AutoTranspose'], current['SingleInstance'], current['bit'],
+                              _copy=False, _widen=False)
+        n, mm = raw.shape
+        if n * draws < _PREDICT_SUMMARY_MIN_CELLS:
+            return self._normalize(np.array(raw, dtype=np.float64), current['minmax'], current['pillow'],
+                                   current['pillow_type'])
+        ds = _engine().upload_clean(raw, np.zeros(n), lambda column_minmax: self._normalize_bounds(
+            mm, column_minmax, current['minmax'], current['pillow'], current['pillow_type']))
+        return _DeviceInputs(ds)
 
     # ------------------------------------------------------------------------------------------------
     # training hot path (FR:1202-1760)
@@ -794,10 +845,11 @@ class FoKL:
         ds = None
         device_moments = resident      # b / btau defaults from the device's sum(y), sum(y^2) instead of host np.var
         if not resident and default_for_fit['clean'] is True and inputs is not None and data is not None:
-            ds = self._clean_on_device(inputs, data, kwargs_to_clean)
+            cleaned = self._clean_on_device(inputs, data, kwargs_to_clean)
+            if cleaned is not None:
+                ds, device_moments = cleaned
         if ds is not None:
             data = self.data
-            device_moments = True      # large dataset cleaned in HBM: no extra host pass over `data`
         elif not resident:
             failed = False
             if default_for_fit['clean'] is True:

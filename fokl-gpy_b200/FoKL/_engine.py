@@ -17,6 +17,7 @@ import contextlib
 import ctypes
 import math
 import os
+import warnings
 
 import numpy as np
 
@@ -294,11 +295,18 @@ class Engine:
 
     # ------------------------------------------------------------------------------------------------
     def upload(self, inputs, data):
-        """Host numpy (N x M normalised inputs, N or N x 1 data) -> DeviceDataset.  H2D copies + one transpose."""
+        """Host numpy (N x M inputs, N or N x 1 data) -> DeviceDataset.  H2D copies + one transpose.  float32 inputs
+        are widened (exactly) and column-major ones (a transposed view, a pandas frame's block) transposed on the
+        device, so neither costs a host pass."""
         torch = self.torch
-        inputs = np.ascontiguousarray(inputs, dtype=np.float64)
+        inputs = np.asarray(inputs)
         if inputs.ndim == 1:
             inputs = inputs[:, None]
+        if inputs.dtype not in (np.float32, np.float64):
+            inputs = np.asarray(inputs, dtype=np.float64)
+        column_major = not inputs.flags.c_contiguous and inputs.flags.f_contiguous
+        if not column_major:
+            inputs = np.ascontiguousarray(inputs)
         data = np.ascontiguousarray(np.asarray(data, dtype=np.float64).reshape(-1))
         n, m = inputs.shape
         if data.shape[0] != n:
@@ -306,27 +314,31 @@ class Engine:
         ldx = _round_up(max(n, 1), 16)
         x = torch.zeros((m, ldx), dtype=torch.float64, device=self.device)
         y = torch.zeros((ldx,), dtype=torch.float64, device=self.device)
-        xr = self._h2d(inputs)
-        x[:, :n].copy_(xr.t())
+        if column_major:
+            x[:, :n].copy_(self._h2d(inputs.T))
+        else:
+            x[:, :n].copy_(self._h2d(inputs).t())
         y[:n].copy_(self._h2d(data))
         self.h2d_bytes = inputs.nbytes + data.nbytes
         return DeviceDataset(x, y, n, m, ldx)
 
     def _h2d(self, a):
-        """Contiguous float64 numpy array -> device tensor of the same shape.  Pinned host pages go out as one async DMA.
-        Ordinary (pageable) arrays -- what a user of `FoKL.fit(inputs, data)` passes -- would be staged by the driver
-        through its own small bounce buffer at ~11 GB/s; from 64 MB up they are instead copied by a few host threads
-        into two pinned buffers that alternate, each DMA overlapping the host copy of the next chunk."""
+        """Contiguous float32 / float64 numpy array -> device tensor of the same shape and dtype.  Pinned host pages go
+        out as one async DMA.  Ordinary (pageable) arrays -- what a user of `FoKL.fit(inputs, data)` passes -- would be
+        staged by the driver through its own small bounce buffer at ~11 GB/s; from 64 MB up they are instead copied by a
+        few host threads into two pinned buffers that alternate, each DMA overlapping the host copy of the next chunk."""
         torch = self.torch
-        t = torch.from_numpy(a)
+        with warnings.catch_warnings():
+            warnings.simplefilter('ignore', UserWarning)     # a read-only array (a pandas block) is only read here
+            t = torch.from_numpy(a)
         if a.nbytes < (64 << 20) or t.is_pinned():
             return t.to(self.device, non_blocking=True)
         from concurrent.futures import ThreadPoolExecutor
         flat = a.reshape(-1)
-        out = torch.empty(flat.shape[0], dtype=torch.float64, device=self.device)
-        chunk = (32 << 20) // 8
+        out = torch.empty(flat.shape[0], dtype=t.dtype, device=self.device)
+        chunk = (32 << 20) // a.itemsize
         if getattr(self, '_bounce', None) is None:
-            self._bounce = [torch.empty(chunk, dtype=torch.float64).pin_memory() for _ in range(2)]
+            self._bounce = [torch.empty((32 << 20) // 8, dtype=torch.float64).pin_memory() for _ in range(2)]
             self._bounce_pool = ThreadPoolExecutor(max_workers=max(2, min(8, (os.cpu_count() or 4) // 2)))
             self._bounce_events = [None, None]
         pool, nthr = self._bounce_pool, self._bounce_pool._max_workers
@@ -336,11 +348,12 @@ class Engine:
             b = k & 1
             if events[b] is not None:
                 events[b].synchronize()                 # the DMA that last read this buffer is done
-            dst = self._bounce[b].numpy()
+            bounce = self._bounce[b].view(t.dtype)
+            dst = bounce.numpy()
             step = -(-(hi - lo) // nthr)
             list(pool.map(lambda r: np.copyto(dst[r:min(r + step, hi - lo)], flat[lo + r:min(lo + r + step, hi)]),
                           range(0, hi - lo, step)))
-            out[lo:hi].copy_(self._bounce[b][:hi - lo], non_blocking=True)
+            out[lo:hi].copy_(bounce[:hi - lo], non_blocking=True)
             events[b] = torch.cuda.Event()
             events[b].record(torch.cuda.current_stream(self.device))
         return out.view(*a.shape)
@@ -370,6 +383,25 @@ class Engine:
             raise ValueError("Input 'minmax' must correspond to input variables (i.e., columns of 'inputs').")
         self._ck(self.lib.fokl_normalize(self.ctx, ds.x.data_ptr(), n, ds.ldx, m, flat.ctypes.data))
         return ds
+
+    def rows_compact(self, ds, keep):
+        """DeviceDataset of the rows of `ds` where the host bool vector `keep` (N) is True, in ascending row order --
+        `inputs[keep, :]`, `data[keep]` -- formed in HBM by fokl_rows_compact; only the N mask bytes cross the bus."""
+        torch = self.torch
+        keep = np.ascontiguousarray(keep, dtype=np.bool_)
+        if keep.shape != (ds.n,):
+            raise ValueError("keep must be a boolean vector with one entry per row")
+        n_keep = int(np.count_nonzero(keep))
+        ldx = _round_up(max(n_keep, 1), 16)
+        mask = torch.from_numpy(keep.view(np.uint8)).to(self.device)
+        x = torch.empty((ds.m, ldx), dtype=torch.float64, device=self.device)
+        y = torch.empty((ldx,), dtype=torch.float64, device=self.device)
+        n_out = ctypes.c_int64(-1)
+        self._ck(self.lib.fokl_rows_compact(self.ctx, ds.x.data_ptr(), ds.y.data_ptr(), ds.n, ds.ldx, ds.m,
+                                            mask.data_ptr(), x.data_ptr(), y.data_ptr(), ldx, ctypes.byref(n_out)))
+        if n_out.value != n_keep:
+            raise RuntimeError("fokl_rows_compact kept %d rows, expected %d" % (n_out.value, n_keep))
+        return DeviceDataset(x, y, n_keep, ds.m, ldx)
 
     def begin_fit(self, ds):
         """Bind a dataset; allocate X (ones column) and the Gram state; compute the data moments."""

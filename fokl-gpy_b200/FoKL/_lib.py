@@ -14,7 +14,7 @@ if os.environ.get('FOKL_B200_LIB'):        # kernel-variant experiments (tools/)
 SOURCES = ['ctx.cu', 'basis.cu', 'gram.cu', 'candidates.cu', 'nested.cu', 'update.cu', 'predict.cu']
 HEADERS = ['fokl_ctx.cuh', 'fokl_math.cuh', 'cand_math.cuh', 'gram_plan.h', 'eigbig.cuh', 'killbig.cuh', 'update_math.cuh', 'predict_math.cuh']
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 KERNEL_CUBIC, KERNEL_BERNOULLI = 0, 1
 RNG_NONE, RNG_INJECTED, RNG_PHILOX = 0, 1, 2
 ERANGE = -4
@@ -89,6 +89,7 @@ PROTOTYPES = {
                                   _i32, _vp]),
     'fokl_column_minmax': (_i32, [_vp, _vp, _i64, _i64, _i32, _vp]),
     'fokl_normalize': (_i32, [_vp, _vp, _i64, _i64, _i32, _vp]),
+    'fokl_rows_compact': (_i32, [_vp, _vp, _vp, _i64, _i64, _i32, _vp, _vp, _vp, _i64, ctypes.POINTER(_i64)]),
 }
 
 _lib = None

@@ -581,15 +581,170 @@ __global__ void normalize_kernel(double *__restrict__ x, int64_t n, int64_t ldx,
 extern "C" int fokl_normalize(fokl_ctx *ctx, double *x, int64_t n, int64_t ldx, int m, const double *minmax)
 {
     FOKL_CHECK_CTX(ctx);
-    if (!x || !minmax || n < 1 || m < 1 || m > 32 || ldx < n) FOKL_FAIL(ctx, FOKL_EINVAL, "normalize: bad argument (m <= 32)");
+    if (!x || !minmax || n < 1 || m < 1 || ldx < n) FOKL_FAIL(ctx, FOKL_EINVAL, "normalize: bad argument");
     int rc = fokl_bind_device(ctx);
     if (rc) return rc;
-    MinMaxArg mm;
-    memset(&mm, 0, sizeof mm);
-    for (int k = 0; k < 2 * m; ++k) mm.v[k] = minmax[k];
     int blocks = (int)((n + 255) / 256);
     if (blocks > ctx->num_sms * 8) blocks = ctx->num_sms * 8;
-    normalize_kernel<<<dim3(blocks, m), 256, 0, ctx->stream>>>(x, n, ldx, mm);
+    // the bounds travel by value, 32 columns per launch: any number of inputs without a device copy of the bounds
+    for (int k0 = 0; k0 < m; k0 += 32) {
+        int mk = m - k0 < 32 ? m - k0 : 32;
+        MinMaxArg mm;
+        memset(&mm, 0, sizeof mm);
+        for (int k = 0; k < 2 * mk; ++k) mm.v[k] = minmax[2 * k0 + k];
+        normalize_kernel<<<dim3(blocks, mk), 256, 0, ctx->stream>>>(x + (int64_t)k0 * ldx, n, ldx, mm);
+        FOKL_LAUNCH_CHECK(ctx);
+    }
+    return FOKL_OK;
+}
+
+// train split (FR:532-542 `inputs[trainlog, :]`): count / scan / scatter over tiles of kCompactTile rows --------------
+// The kept count is needed on the host before anything is written (ldx_out is checked against it and n_out returned),
+// so the count is its own pass; the scatter then re-reads the tile's mask bytes (N bytes against 8 N (m + 1) of values).
+static constexpr int kCompactThreads = 256;
+static constexpr int kCompactPer = 16;                                   // rows per thread and tile pass
+static constexpr int kCompactTile = kCompactThreads * kCompactPer;       // 4096 rows per block
+
+__global__ void __launch_bounds__(kCompactThreads) rows_compact_count(const uint8_t *__restrict__ keep, int64_t n,
+                                                                      int64_t *__restrict__ tile_count)
+{
+    int64_t base = (int64_t)blockIdx.x * kCompactTile;
+    int c = 0;
+#pragma unroll
+    for (int r = 0; r < kCompactPer; ++r) {
+        int64_t i = base + r * kCompactThreads + threadIdx.x;
+        c += (i < n && keep[i]) ? 1 : 0;
+    }
+    for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
+    __shared__ int warp_c[kCompactThreads / 32];
+    if ((threadIdx.x & 31) == 0) warp_c[threadIdx.x >> 5] = c;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        int t = 0;
+        for (int w = 0; w < kCompactThreads / 32; ++w) t += warp_c[w];
+        tile_count[blockIdx.x] = t;
+    }
+}
+
+// exclusive scan of the tile counts in place (one block); total -> *total
+__global__ void __launch_bounds__(1024) rows_compact_scan(int64_t *__restrict__ tile_off, int64_t tiles,
+                                                          int64_t *__restrict__ total)
+{
+    __shared__ int64_t warp_s[32];
+    __shared__ int64_t carry;
+    if (threadIdx.x == 0) carry = 0;
+    __syncthreads();
+    int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int64_t b0 = 0; b0 < tiles; b0 += 1024) {
+        int64_t i = b0 + threadIdx.x;
+        int64_t v = i < tiles ? tile_off[i] : 0, s = v;
+        for (int o = 1; o < 32; o <<= 1) {
+            int64_t t = __shfl_up_sync(0xffffffffu, s, o);
+            if (lane >= o) s += t;
+        }
+        if (lane == 31) warp_s[warp] = s;
+        __syncthreads();
+        if (warp == 0) {
+            int64_t w = warp_s[lane];
+            for (int o = 1; o < 32; o <<= 1) {
+                int64_t t = __shfl_up_sync(0xffffffffu, w, o);
+                if (lane >= o) w += t;
+            }
+            warp_s[lane] = w;                                            // inclusive over warps
+        }
+        __syncthreads();
+        int64_t incl = s + (warp > 0 ? warp_s[warp - 1] : 0) + carry;
+        if (i < tiles) tile_off[i] = incl - v;
+        __syncthreads();
+        if (threadIdx.x == 1023) carry = incl;
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) *total = carry;
+}
+
+// one tile per block: each thread's kCompactPer rows get their output position (or -1) from warp ballots and a scan
+// of the warp totals, then every column (x's m, then y) is copied through those positions
+__global__ void __launch_bounds__(kCompactThreads) rows_compact_scatter(
+    const double *__restrict__ x, const double *__restrict__ y, int64_t n, int64_t ldx, int m,
+    const uint8_t *__restrict__ keep, const int64_t *__restrict__ tile_off, double *__restrict__ x_out,
+    double *__restrict__ y_out, int64_t ldx_out)
+{
+    __shared__ int warp_c[kCompactThreads / 32];
+    int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int64_t base = (int64_t)blockIdx.x * kCompactTile;
+    int64_t out0 = tile_off[blockIdx.x];
+    int off = 0;
+    int pos[kCompactPer];                                                // position within the tile's output run
+#pragma unroll
+    for (int r = 0; r < kCompactPer; ++r) {
+        int64_t i = base + r * kCompactThreads + threadIdx.x;
+        bool k = i < n && keep[i];
+        unsigned bal = __ballot_sync(0xffffffffu, k);
+        if (lane == 0) warp_c[warp] = __popc(bal);
+        __syncthreads();
+        int before = 0, all = 0;
+#pragma unroll
+        for (int w = 0; w < kCompactThreads / 32; ++w) {
+            int c = warp_c[w];
+            before += w < warp ? c : 0;
+            all += c;
+        }
+        pos[r] = k ? off + before + __popc(bal & ((1u << lane) - 1u)) : -1;
+        off += all;
+        __syncthreads();
+    }
+    for (int c = 0; c <= m; ++c) {
+        const double *src = c < m ? x + (int64_t)c * ldx : y;
+        double *dst = (c < m ? x_out + (int64_t)c * ldx_out : y_out) + out0;
+#pragma unroll
+        for (int r = 0; r < kCompactPer; ++r) {
+            int64_t i = base + r * kCompactThreads + threadIdx.x;
+            if (pos[r] >= 0) dst[pos[r]] = src[i];
+        }
+    }
+}
+
+// rows [n_out, ldx_out) of every output column and of y_out = 0.0 (Engine.upload's padding)
+__global__ void rows_compact_pad(double *__restrict__ x_out, double *__restrict__ y_out, int m, int64_t n_out,
+                                 int64_t ldx_out)
+{
+    int c = blockIdx.y;
+    double *dst = c < m ? x_out + (int64_t)c * ldx_out : y_out;
+    for (int64_t i = n_out + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < ldx_out;
+         i += (int64_t)gridDim.x * blockDim.x)
+        dst[i] = 0.0;
+}
+
+extern "C" int fokl_rows_compact(fokl_ctx *ctx, const double *x, const double *y, int64_t n, int64_t ldx, int m,
+                                 const uint8_t *keep, double *x_out, double *y_out, int64_t ldx_out, int64_t *n_out)
+{
+    FOKL_CHECK_CTX(ctx);
+    if (!x || !y || !keep || !x_out || !y_out || !n_out || n < 1 || m < 1 || ldx < n || ldx_out < 0)
+        FOKL_FAIL(ctx, FOKL_EINVAL, "rows_compact: bad argument");
+    int rc = fokl_bind_device(ctx);
+    if (rc) return rc;
+    int64_t tiles = (n + kCompactTile - 1) / kCompactTile;
+    if (tiles > 0x7fffffffLL) FOKL_FAIL(ctx, FOKL_EINVAL, "rows_compact: n too large");
+    int64_t *scr = (int64_t *)fokl_scratch(ctx, fokl_ctx::B_MISC, (size_t)(tiles + 1) * sizeof(int64_t));
+    if (!scr) return FOKL_ENOMEM;
+    rows_compact_count<<<(unsigned)tiles, kCompactThreads, 0, ctx->stream>>>(keep, n, scr);
     FOKL_LAUNCH_CHECK(ctx);
+    rows_compact_scan<<<1, 1024, 0, ctx->stream>>>(scr, tiles, scr + tiles);
+    FOKL_LAUNCH_CHECK(ctx);
+    int64_t kept = 0;
+    FOKL_CUDA(ctx, cudaMemcpyAsync(&kept, scr + tiles, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    FOKL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (ldx_out < kept) FOKL_FAIL(ctx, FOKL_EINVAL, "rows_compact: ldx_out below the kept row count");
+    rows_compact_scatter<<<(unsigned)tiles, kCompactThreads, 0, ctx->stream>>>(x, y, n, ldx, m, keep, scr, x_out,
+                                                                               y_out, ldx_out);
+    FOKL_LAUNCH_CHECK(ctx);
+    if (ldx_out > kept) {
+        int64_t pad = ldx_out - kept;
+        int blocks = (int)((pad + 255) / 256);
+        if (blocks > ctx->num_sms * 4) blocks = ctx->num_sms * 4;
+        rows_compact_pad<<<dim3(blocks, m + 1), 256, 0, ctx->stream>>>(x_out, y_out, m, kept, ldx_out);
+        FOKL_LAUNCH_CHECK(ctx);
+    }
+    *n_out = kept;
     return FOKL_OK;
 }

@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define FOKL_ABI_VERSION 2
+#define FOKL_ABI_VERSION 3
 
 #define FOKL_OK 0
 #define FOKL_EINVAL (-1)   /* bad argument                                  */
@@ -299,9 +299,18 @@ int fokl_deriv_summary(fokl_ctx *ctx, int kernel, const double *x, int64_t ldx, 
 
 /* clean/_normalize on device (FR:377, 436-437): minmax_out (dev, 2*m) = per-column min, max of x
  * (column-major n x m, ldx); then fokl_normalize applies x = (x - min) / (max - min) in place with
- * minmax (host, 2*m). */
+ * minmax (host, 2*m), for any m >= 1. */
 int fokl_column_minmax(fokl_ctx *ctx, const double *x, int64_t n, int64_t ldx, int m, double *minmax_out);
 int fokl_normalize(fokl_ctx *ctx, double *x, int64_t n, int64_t ldx, int m, const double *minmax);
+
+/* train split of clean (FR:532-542, `inputs[trainlog, :]`, `data[trainlog]`): the rows i < n with keep[i] != 0
+ * (dev, n bytes) of x (dev, column-major [m][ldx]) and y (dev, n) are written in ascending row order to x_out
+ * (dev, [m][ldx_out]) and y_out (dev, ldx_out); rows [*n_out, ldx_out) of every output column and of y_out are set to
+ * 0.0.  *n_out (host) = kept row count.  The outputs must not overlap the inputs.  Synchronises the context's stream
+ * once (the kept count).  A null pointer, n < 1, m < 1, ldx < n or ldx_out below the kept count returns FOKL_EINVAL
+ * before anything is written to the outputs. */
+int fokl_rows_compact(fokl_ctx *ctx, const double *x, const double *y, int64_t n, int64_t ldx, int m,
+                      const uint8_t *keep, double *x_out, double *y_out, int64_t ldx_out, int64_t *n_out);
 
 #ifdef __cplusplus
 }
