@@ -72,6 +72,9 @@ _DERIV_CHUNK_BYTES = 256 << 20
 # `clean` (fit(clean=True), evaluate(inputs, clean=True)) formats, normalises and splits the dataset in HBM once the raw
 # inputs have at least this many cells; smaller datasets take the host path, where the pass over them costs little
 _CLEAN_ON_DEVICE_MIN_CELLS = 1 << 20
+# generate_trainlog draws its split in HBM (fokl_trainlog: the host loop's mask and numpy RNG end state, bit for bit)
+# from this many rows, wherever the dataset is cleaned; below it the host loop costs little
+_TRAINLOG_ON_DEVICE_MIN_ROWS = 1 << 20
 
 
 def _engine(device=None):
@@ -169,6 +172,38 @@ def _column_minmax_host(inputs):
     except ImportError:
         pass
     return bounds
+
+
+def _have_cuda():
+    try:
+        import torch
+        return torch.cuda.is_available()
+    except ImportError:
+        return False
+
+
+def _device_trainlog(train, n):
+    """`generate_trainlog(train, n)`'s mask as a device uint8 tensor, drawn by fokl_trainlog from the legacy numpy RNG,
+    whose state it then advances exactly as the host loop would (has_gauss / cached_gaussian are left as they were).
+    None when the split is not drawn on the device: train >= 1, n below _TRAINLOG_ON_DEVICE_MIN_ROWS or at least 2^31,
+    or no CUDA device."""
+    if not (train < 1 and _TRAINLOG_ON_DEVICE_MIN_ROWS <= n < (1 << 31) and _have_cuda()):
+        return None
+    state = np.random.get_state()
+    keep, key, pos, _ = _engine().trainlog(state[1], state[2], n, max(int(n * train), 2))
+    np.random.set_state((state[0], key, pos, state[3], state[4]))
+    return keep
+
+
+def _dist_world():
+    """torch.distributed when it is initialised with more than one rank, else None."""
+    try:
+        import torch.distributed as dist
+    except ImportError:
+        return None
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+        return dist
+    return None
 
 
 class _DeviceInputs:
@@ -425,7 +460,7 @@ class FoKL:
             # (the reference's capping of values outside [0, 1] is dead code -- `np.max(...) is True`, FR:488)
 
         if hasattr(self, 'inputs') is False or _setattr is True:
-            trainlog = self.generate_trainlog(current['train'], inputs.shape[0])
+            trainlog, _ = self._shard_trainlog(current['train'], inputs.shape[0])
             self.inputs, self.data, self.trainlog = inputs, data, trainlog
 
         if data is None:
@@ -437,6 +472,9 @@ class FoKL:
         if train < 1:
             if n is None:
                 n = self.inputs.shape[0]
+            keep = _device_trainlog(train, n)
+            if keep is not None:
+                return keep.cpu().numpy().view(bool)
             l_log = max(int(n * train), 2)
             idx = np.array([], dtype=int)
             while len(idx) < l_log:
@@ -448,6 +486,40 @@ class FoKL:
             trainlog[idx] = True
             return trainlog
         return None
+
+    def _shard_trainlog(self, train, n):
+        """`generate_trainlog(train, n)` for the n rows `clean` was given: (host bool mask or None, the same mask as a
+        device uint8 tensor when it was drawn there, else None).  Under torch.distributed every rank holds a row shard
+        of one dataset, in rank order: the shard sizes are gathered, rank 0's numpy RNG state is broadcast, every rank
+        draws the split of all N rows (in HBM from _TRAINLOG_ON_DEVICE_MIN_ROWS rows on, as a single process would) and
+        keeps its own rows.  So the shards' masks concatenate to the single-process mask, and every rank's RNG ends in
+        the single process's state."""
+        if not train < 1:
+            return None, None
+        dist = _dist_world()
+        lo, total = 0, n
+        if dist is not None:
+            import torch
+            dev = torch.device('cuda', torch.cuda.current_device()) if dist.get_backend() == 'nccl' else torch.device('cpu')
+            mine = torch.tensor([n], dtype=torch.int64, device=dev)
+            sizes = [torch.zeros_like(mine) for _ in range(dist.get_world_size())]
+            dist.all_gather(sizes, mine)
+            sizes = [int(t.item()) for t in sizes]
+            lo, total = sum(sizes[:dist.get_rank()]), sum(sizes)
+            st = np.random.get_state()
+            packed = np.concatenate([np.asarray(st[1], dtype=np.int64), [st[2], st[3]],
+                                     np.array([st[4]], dtype=np.float64).view(np.int64)])
+            t = torch.from_numpy(packed).to(dev)
+            dist.broadcast(t, src=0)
+            packed = t.cpu().numpy()
+            np.random.set_state(('MT19937', packed[:624].astype(np.uint32), int(packed[624]), int(packed[625]),
+                                 float(packed[626:627].view(np.float64)[0])))
+        keep = _device_trainlog(train, total)
+        if keep is None:
+            mask = self.generate_trainlog(train, total)
+            return (mask if dist is None else mask[lo:lo + n].copy()), None
+        keep = keep[lo:lo + n]
+        return keep.cpu().numpy().view(bool), keep
 
     def trainset(self):
         """Train inputs and data after `clean` (FR:532-542)."""
@@ -759,7 +831,8 @@ class FoKL:
         """`clean` for `fit(clean=True)` done in HBM (FR:248-542): `_format`'s checks and warnings run on the host
         unchanged, but the raw inputs go to the device as they are (float32 widened, a column-major block transposed
         there), the per-column min / max and (x - min) / (max - min) run there (bit-identical to the host expression),
-        and a train split (`generate_trainlog` on the host, unchanged) keeps its rows with fokl_rows_compact.  Sets
+        and a train split (`_shard_trainlog`; a mask drawn in HBM goes to the kernel as it is) keeps its rows with
+        fokl_rows_compact.  Sets
         `inputs` (the train rows, materialised on the host only if somebody reads them), `data` (the train rows) and
         `trainlog` as the host path's `fit` leaves them.  Returns (DeviceDataset of the train rows, moments_on_device)
         or None when the request needs the host path (_device_raw_inputs).  moments_on_device: the b / btau defaults
@@ -780,9 +853,10 @@ class FoKL:
         eng = _engine()
         ds = eng.upload_clean(raw, data, lambda column_minmax: self._normalize_bounds(
             mm, column_minmax, current['minmax'], current['pillow'], current['pillow_type']))
-        trainlog = self.generate_trainlog(current['train'], n)
+        trainlog, keep = self._shard_trainlog(current['train'], n)
         if trainlog is not None:
-            ds = eng.rows_compact(ds, trainlog)
+            ds = eng.rows_compact(ds, trainlog) if keep is None else \
+                eng.rows_compact(ds, keep, int(np.count_nonzero(trainlog)))
             data = data[trainlog]
         self.__dict__['inputs'] = _DeviceInputs(ds)
         self.data = data

@@ -384,16 +384,25 @@ class Engine:
         self._ck(self.lib.fokl_normalize(self.ctx, ds.x.data_ptr(), n, ds.ldx, m, flat.ctypes.data))
         return ds
 
-    def rows_compact(self, ds, keep):
+    def rows_compact(self, ds, keep, n_keep=None):
         """DeviceDataset of the rows of `ds` where the host bool vector `keep` (N) is True, in ascending row order --
-        `inputs[keep, :]`, `data[keep]` -- formed in HBM by fokl_rows_compact; only the N mask bytes cross the bus."""
+        `inputs[keep, :]`, `data[keep]` -- formed in HBM by fokl_rows_compact; only the N mask bytes cross the bus.
+        `keep` may instead be a device uint8 / bool tensor of N entries (fokl_trainlog's mask), with its count of
+        nonzero entries in n_keep; then nothing crosses the bus."""
         torch = self.torch
-        keep = np.ascontiguousarray(keep, dtype=np.bool_)
-        if keep.shape != (ds.n,):
-            raise ValueError("keep must be a boolean vector with one entry per row")
-        n_keep = int(np.count_nonzero(keep))
+        if isinstance(keep, torch.Tensor):
+            if keep.shape != (ds.n,) or keep.dtype not in (torch.uint8, torch.bool) or keep.device != ds.x.device \
+                    or not keep.is_contiguous() or n_keep is None:
+                raise ValueError("a device keep mask must be a contiguous uint8 / bool tensor with one entry per row, "
+                                 "beside the dataset, and come with its count")
+            n_keep, mask = int(n_keep), keep
+        else:
+            keep = np.ascontiguousarray(keep, dtype=np.bool_)
+            if keep.shape != (ds.n,):
+                raise ValueError("keep must be a boolean vector with one entry per row")
+            n_keep = int(np.count_nonzero(keep))
+            mask = torch.from_numpy(keep.view(np.uint8)).to(self.device)
         ldx = _round_up(max(n_keep, 1), 16)
-        mask = torch.from_numpy(keep.view(np.uint8)).to(self.device)
         x = torch.empty((ds.m, ldx), dtype=torch.float64, device=self.device)
         y = torch.empty((ldx,), dtype=torch.float64, device=self.device)
         n_out = ctypes.c_int64(-1)
@@ -402,6 +411,20 @@ class Engine:
         if n_out.value != n_keep:
             raise RuntimeError("fokl_rows_compact kept %d rows, expected %d" % (n_out.value, n_keep))
         return DeviceDataset(x, y, n_keep, ds.m, ldx)
+
+    def trainlog(self, key, pos, n, l_log):
+        """`generate_trainlog`'s split of n rows (l_log = max(int(n * train), 2)) drawn in HBM by fokl_trainlog from the
+        legacy MT19937 state (key[624], pos): (device uint8 keep-mask of n entries, key and pos after the last word the
+        host loop consumes, words consumed)."""
+        key = np.ascontiguousarray(key, dtype=np.uint32)
+        if key.shape != (624,):
+            raise ValueError("key must hold the 624 words of an MT19937 state")
+        keep = self.torch.empty(int(n), dtype=self.torch.uint8, device=self.device)
+        key_out = np.empty(624, dtype=np.uint32)
+        pos_out, words = ctypes.c_int(-1), ctypes.c_int64(-1)
+        self._ck(self.lib.fokl_trainlog(self.ctx, key.ctypes.data, int(pos), int(n), int(l_log), keep.data_ptr(),
+                                        key_out.ctypes.data, ctypes.byref(pos_out), ctypes.byref(words)))
+        return keep, key_out, pos_out.value, words.value
 
     def begin_fit(self, ds):
         """Bind a dataset; allocate X (ones column) and the Gram state; compute the data moments."""

@@ -11,10 +11,10 @@ CSRC = os.path.join(os.path.dirname(_HERE), 'csrc')
 SO_PATH = os.path.join(CSRC, 'libfokl_b200.so')
 if os.environ.get('FOKL_B200_LIB'):        # kernel-variant experiments (tools/): another build of the same sources
     SO_PATH = os.path.abspath(os.environ['FOKL_B200_LIB'])
-SOURCES = ['ctx.cu', 'basis.cu', 'gram.cu', 'candidates.cu', 'nested.cu', 'update.cu', 'predict.cu']
-HEADERS = ['fokl_ctx.cuh', 'fokl_math.cuh', 'cand_math.cuh', 'gram_plan.h', 'eigbig.cuh', 'killbig.cuh', 'update_math.cuh', 'predict_math.cuh']
+SOURCES = ['ctx.cu', 'basis.cu', 'gram.cu', 'candidates.cu', 'nested.cu', 'update.cu', 'predict.cu', 'trainlog.cu']
+HEADERS = ['fokl_ctx.cuh', 'fokl_math.cuh', 'cand_math.cuh', 'gram_plan.h', 'eigbig.cuh', 'killbig.cuh', 'update_math.cuh', 'predict_math.cuh', 'trainlog_math.cuh']
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 KERNEL_CUBIC, KERNEL_BERNOULLI = 0, 1
 RNG_NONE, RNG_INJECTED, RNG_PHILOX = 0, 1, 2
 ERANGE = -4
@@ -90,6 +90,7 @@ PROTOTYPES = {
     'fokl_column_minmax': (_i32, [_vp, _vp, _i64, _i64, _i32, _vp]),
     'fokl_normalize': (_i32, [_vp, _vp, _i64, _i64, _i32, _vp]),
     'fokl_rows_compact': (_i32, [_vp, _vp, _vp, _i64, _i64, _i32, _vp, _vp, _vp, _i64, ctypes.POINTER(_i64)]),
+    'fokl_trainlog': (_i32, [_vp, _vp, _i32, _i64, _i64, _vp, _vp, ctypes.POINTER(_i32), ctypes.POINTER(_i64)]),
 }
 
 _lib = None

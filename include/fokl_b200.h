@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define FOKL_ABI_VERSION 3
+#define FOKL_ABI_VERSION 4
 
 #define FOKL_OK 0
 #define FOKL_EINVAL (-1)   /* bad argument                                  */
@@ -311,6 +311,17 @@ int fokl_normalize(fokl_ctx *ctx, double *x, int64_t n, int64_t ldx, int m, cons
  * before anything is written to the outputs. */
 int fokl_rows_compact(fokl_ctx *ctx, const double *x, const double *y, int64_t n, int64_t ldx, int m,
                       const uint8_t *keep, double *x_out, double *y_out, int64_t ldx_out, int64_t *n_out);
+
+/* train split of clean (FR:509-530 `generate_trainlog(train, n)`), bit for bit with numpy's legacy RandomState: from
+ * the MT19937 state key[624] (host) / pos (0 .. 624), with l_log = max(int(n * train), 2) computed by the caller,
+ * keep (dev, n bytes) = 1 for the rows the reference's mask keeps and 0 elsewhere; key_out[624] / *pos_out (host) = the
+ * state after the last word the reference consumes (np.random.set_state(('MT19937', key_out, *pos_out, has_gauss,
+ * cached_gaussian)) leaves numpy where generate_trainlog would); *words_out = words consumed.  Synchronises the
+ * context's stream.  Device memory: about n / 8 + 12 n bytes plus a 41 MB word window, allocated and freed within the
+ * call.  A null pointer, pos outside [0, 624] or l_log outside [2, n], n >= 2^31 returns FOKL_EINVAL before anything
+ * is written to the outputs. */
+int fokl_trainlog(fokl_ctx *ctx, const uint32_t *key, int pos, int64_t n, int64_t l_log, uint8_t *keep,
+                  uint32_t *key_out, int *pos_out, int64_t *words_out);
 
 #ifdef __cplusplus
 }
